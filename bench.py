@@ -93,7 +93,15 @@ def parse():
     p.add_argument("--only-modes", action="store_true", help="skip the headline measurement (profiling the --modes blocks)")
     p.add_argument("--mode-steps", type=int, default=0, help="timed steps of the --modes blocks (0 = min(--steps, 5))")
     p.add_argument("--max-rows", type=int, default=1 << 22, help="rows per shard of the streamed forward (--modes blocks)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write the last step's logits for a fixed sample of the nodes to DIR/logits.npy "
+                        "(float32 [rows, C], node order) and their node ids to DIR/node_ids.npy (float64), for comparing builds")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "ours" or a.gpus != 1 or a.only_modes):
+        p.error("--dump-outputs takes the headline of a single-GPU --impl ours run")
+    return a
 
 
 def workload_shape(name):
@@ -154,6 +162,22 @@ def measured_peaks():
         d = json.load(open(path))
         return d.get("hbm_gbs", 6650.0), d.get("bf16_tflops_sustained", 1400.0), "measured"
     return 6650.0, 1590.0, "fallback"
+
+
+DUMP_ROWS = 1 << 18  # nodes in --dump-outputs: 262,144 x (47 fp32 logits + an fp64 id) = 51 MB, under the 64 MB a dump may take
+
+
+def dump_outputs(out_dir, logits, core_gid, n):
+    """--dump-outputs: rows of `logits` ([n_core, C], pack order, core_gid[i] = node of row i) for a seeded sample of the n
+    nodes (all of them when n <= DUMP_ROWS), in ascending node order.  Keyed by node id, so a build that orders the pack
+    differently still compares row for row."""
+    ids = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+    row_of_node = torch.empty(n, dtype=torch.long, device=logits.device)
+    row_of_node[core_gid.long()] = torch.arange(core_gid.numel(), device=logits.device)
+    sample = logits[row_of_node[torch.from_numpy(ids).to(logits.device)]].float().cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "logits.npy"), sample)
+    np.save(os.path.join(out_dir, "node_ids.npy"), ids.astype(np.float64))
 
 
 def generate(args, device):
@@ -917,6 +941,8 @@ def main_ours(args):
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms = float(t.item())
+    if args.dump_outputs:  # single GPU (parse): `out` is the last timed step's [n, C] logits in pack order
+        dump_outputs(args.dump_outputs, out, pack.core_gid, n)
 
     # ---- N > 1: the result equals a single-GPU forward of the whole pack on EVERY rank (outside the timing).  Sharded
     # outputs are all-gathered once here for the check; the gathered variants are checked as they come out of a step.

@@ -663,3 +663,33 @@ def test_pack_builder_edgeless_graph(fg, mode):
     out, ids = fg.infer.node_infer_Gs(sd, pack, X.to(dev()))
     want = fo.classify_node(sd, X[:n], torch.zeros(2, 0, dtype=torch.long))  # isolated nodes: out = lin(x) + b
     assert_close(out.detach().cpu().numpy(), want.numpy()[ids.cpu().numpy()])
+
+
+def test_bench_dump_outputs_repeats_run_to_run(tmp_path):
+    """`bench.py --dump-outputs DIR` on the small workload: the last timed step's logits (log_softmax rows, float32, keyed by
+    float64 node ids, under 64 MB in all) come out the same from two runs with the same arguments, which is what makes two
+    builds comparable output for output."""
+    import json
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    dumps = []
+    for run in ("a", "b"):
+        d = tmp_path / run
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--workload", "products-small", "--steps", "2",
+                              "--warmup", "1", "--modes=", "--no-cpu-baseline", "--no-projection", "--no-e2e",
+                              "--dump-outputs", str(d)], capture_output=True, text=True, timeout=600, cwd=root)
+        assert out.returncode == 0, out.stderr[-2000:]
+        assert json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])["steps"] == 2
+        assert sorted(os.listdir(d)) == ["logits.npy", "node_ids.npy"]
+        assert sum(os.path.getsize(d / f) for f in os.listdir(d)) <= 64 << 20
+        dumps.append((np.load(d / "node_ids.npy"), np.load(d / "logits.npy")))
+    (ids, logits), (ids_b, logits_b) = dumps
+    n = 200000  # products-small: every node fits the sample
+    assert ids.dtype == np.float64 and np.array_equal(ids, np.arange(n))
+    assert logits.dtype == np.float32 and logits.shape == (n, 47) and np.isfinite(logits).all()
+    lse = np.log(np.exp(logits.astype(np.float64)).sum(1))
+    assert np.abs(lse).max() < 1e-4
+    assert np.array_equal(ids, ids_b)
+    assert np.abs(logits - logits_b).max() <= 1e-5 * max(1.0, float(np.abs(logits).max()))

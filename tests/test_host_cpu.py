@@ -162,6 +162,18 @@ def test_bench_reference_arm_contract_on_cpu():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+@pytest.mark.parametrize("flags", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "d"],
+                                   ["--gpus", "2", "--dump-outputs", "d"], ["--only-modes", "--dump-outputs", "d"]])
+def test_bench_refuses_arguments_it_cannot_honour(tmp_path, flags):
+    """No timed step, or a dump of a run whose timed path is not the single-GPU headline: a usage error before any work."""
+    import subprocess
+    import sys
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + flags, capture_output=True, text=True, timeout=120,
+                         cwd=tmp_path)
+    assert out.returncode == 2 and "error:" in out.stderr and out.stdout == ""
+    assert os.listdir(tmp_path) == []
+
+
 @pytest.mark.parametrize("mode,flags", [("none", {}), ("extra", dict(extra_node=True)), ("cluster", dict(extra_node=True, cluster_node=True))])
 def test_reference_cache_layout_roundtrip(tmp_path, mode, flags):
     """The reference's preprocessing cache (main.py:131-172 `save()`, read at main.py:270-275 / inference.py:543-548): file
