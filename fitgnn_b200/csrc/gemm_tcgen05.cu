@@ -1022,6 +1022,14 @@ gemm_bf16x3_kernel(const GatherArgs ga, const EpiArgs ea, const __grid_constant_
             bulk_commit();
           }
         } else if (m < M && dest_row >= 0) {
+          // a row map with the pitch N rounded up to 4: the pitch-padding columns [N, ldy) are written as zeros, like the
+          // bulk row copies do, so that what a caller's buffer holds does not depend on which store path ran
+          const int n_end = (ea.row_map && ldy == (int64_t)((N + 3) & ~3)) ? (int)ldy : N;
+          if (n0 + c0 + 32 > N) {
+#pragma unroll
+            for (int j = 0; j < 32; ++j)
+              if (n0 + c0 + j >= N) v[j] = 0.f;
+          }
           const int n_dst = ea.n_peers > 0 ? ea.n_peers : 1;
 #pragma unroll
           for (int p = 0; p < 8; ++p) {
@@ -1029,12 +1037,12 @@ gemm_bf16x3_kernel(const GatherArgs ga, const EpiArgs ea, const __grid_constant_
             float* yp = ea.n_peers > 0 ? ea.peers[p] + dest_row * ldy + n0 : yrow;
 #pragma unroll
             for (int j = 0; j < 32; j += 4) {
-              if (vec_ok && j + 4 <= box_cols && n0 + c0 + j + 4 <= N) {
+              if (vec_ok && j + 4 <= box_cols && n0 + c0 + j + 4 <= n_end) {
                 *reinterpret_cast<float4*>(yp + c0 + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
               } else {
 #pragma unroll
                 for (int u = 0; u < 4; ++u)
-                  if (j + u < box_cols && n0 + c0 + j + u < N) yp[c0 + j + u] = v[j + u];
+                  if (j + u < box_cols && n0 + c0 + j + u < n_end) yp[c0 + j + u] = v[j + u];
               }
             }
           }

@@ -302,7 +302,9 @@ int fitgnn_gemm_rowscale_bias_act_split(int precision, const void* A, const void
  * (PackedForward(precision="fp16") for the hidden -> hidden transforms): one MMA per k-step, 2^-11 per element on both
  * operands (measured end to end: 1.8e-5 of the largest logit against 1.6e-5 with hi/lo weights, profiles/r2_precision_study.md),
  * and for K <= 512 the CTA-pair kernel keeps each CTA's half of the 256-row weight block resident in shared memory
- * (W-stationary pairs: only A streams; tuning switch gemm_pair_ws = 0 restores the streaming plan). */
+ * (W-stationary pairs: only A streams; tuning switch gemm_pair_ws = 0 restores the streaming plan).
+ * Every fp16-plane output of these kernels is rounded to nearest once and saturates: a value beyond +-65504 is stored as
+ * +-65504, never as inf. */
 int fitgnn_split_f16(const float* X, int64_t ldx, int64_t rows, int cols, void* hi, void* lo, int64_t ldo, void* stream);
 int fitgnn_gemm_f16(const void* A, int64_t lda, const void* W_hi, const void* W_lo, int64_t ldw,
                     const float* row_scale, const float* bias, int64_t M, int K, int N, int act, int head,
@@ -317,7 +319,8 @@ int fitgnn_spmm_symnorm_f16(const int32_t* rowptr, const int32_t* col, const flo
  * other lanes), then bias and activation; A and Y are fp16 planes [M, lda] / [M, ldy], W fp16 planes (W_lo may be NULL: one
  * plane).  For K > 128 and M >= 4096 this is the CTA-pair kernel (W-stationary when the weights fit), whose tensor-bound
  * main loop hides the exchange-heavy epilogue; PackedForward(precision="fp16" / "fp16x2") uses it for every layer after the
- * first (schedule: spmm0 -> transform -> [conv]* -> head). */
+ * first (schedule: spmm0 -> transform -> [conv]* -> head).  A padding row (dinv = 0) is NOT written as zeros: it holds
+ * act(bias) rounded to fp16 (0 without a bias), because the trailing dinv[r] scales the aggregate and not the bias. */
 int fitgnn_gcn_conv_aligned_f16(const void* A, int64_t lda, const void* W_hi, const void* W_lo, int64_t ldw,
                                 const float* bias, int64_t M, int K, int N, int act, const uint64_t* agg_desc,
                                 const float* dinv, void* Y, int64_t ldy, void* stream);
@@ -333,7 +336,8 @@ int fitgnn_gcn_transform_aggregate_f16(int in_f16, const void* A_hi, const void*
 /* fitgnn_gemm_bias_act (BF16X3) whose output row m is written to Y row row_map[m] and skipped when row_map[m] < 0:
  * drops the padding rows of an aligned pack / scatters lt1's output (network.py:34-35) straight into the caller's
  * row order.  When ldy is N rounded up to a multiple of 4, the pitch-padding columns [N, ldy) of written rows are
- * zero-filled (narrow heads write whole rows with bulk copies); otherwise they are left untouched. */
+ * zero-filled, whichever store path runs (narrow heads write whole rows with bulk copies, the others per row); otherwise
+ * they are left untouched. */
 int fitgnn_gemm_head_rows(const void* A_hi, const void* A_lo, int64_t lda, const void* W_hi,
                           const void* W_lo, int64_t ldw, const float* bias, int64_t M, int K, int N,
                           int act, int head, const int32_t* row_map, float* Y, int64_t ldy, void* stream);
