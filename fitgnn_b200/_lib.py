@@ -45,12 +45,18 @@ SIGNATURES = {
     "fitgnn_csr_workspace_bytes": (c_size, [c_i64, c_i64]),
     "fitgnn_csr_plan": (c_i32, [c_void, c_i64, c_i64, c_void, c_size, C.POINTER(c_i64), c_void]),
     "fitgnn_csr_fill": (c_i32, [c_i64, c_void, c_size, c_void, c_void, c_void, c_void]),
+    "fitgnn_csr_raw_plan": (c_i32, [c_void, c_i64, c_i64, c_void, c_size, C.POINTER(c_i64), c_void]),
+    "fitgnn_csr_raw_fill": (c_i32, [c_i64, c_void, c_size, c_void, c_void, c_void]),
     "fitgnn_pack_workspace_bytes": (c_size, [c_i64, c_i64, c_i64, c_i32, c_i64]),
     "fitgnn_pack_plan": (c_i32, [c_void, c_i64, c_i64, c_void, c_i64, c_i32, c_void, c_void, c_i64, c_void, c_size,
                                  C.POINTER(PlanStruct), c_void]),
     "fitgnn_pack_fill": (c_i32, [C.POINTER(PlanStruct), C.POINTER(PackStruct), c_void, c_size, c_void, c_size, c_void]),
     "fitgnn_spmm_symnorm": (c_i32, [c_void, c_void, c_void, c_void, c_i64, c_i32, c_void, c_void, c_i32, c_void, c_i64,
                                     c_void, c_void, c_i64, c_void]),
+    "fitgnn_spmm_mean_concat": (c_i32, [c_void, c_void, c_void, c_i64, c_i32, c_i32, c_void, c_void, c_i32, c_void, c_i64,
+                                        c_void, c_void, c_i64, c_void]),
+    "fitgnn_spmm_mean_root": (c_i32, [c_void, c_void, c_void, c_i64, c_i32, c_i64, c_void, c_void, c_i32, c_void, c_i32,
+                                      c_void, c_i64, c_void, c_void, c_i64, c_void]),
     "fitgnn_spmm_symnorm_grouped": (c_i32, [c_void, c_void, c_void, c_void, c_i64, c_i32, c_void, c_i64, c_i32, c_void,
                                             c_void, c_i64, c_i32, C.c_float, c_void]),
     "fitgnn_spmm_symnorm_grouped_f16": (c_i32, [c_void, c_void, c_void, c_void, c_i64, c_i32, c_void, c_i64, c_i32, c_void,

@@ -128,3 +128,95 @@ def gcn_conv(x, weight, bias, csr: CsrPair, act: int = ops.ACT_NONE, dropout_p: 
     if dropout_p > 0.0 and seed is None:
         seed = int(torch.randint(0, 2 ** 62, (1,)).item())
     return GCNConvFn.apply(x, weight, bias, csr, act, float(dropout_p), int(seed or 0))
+
+
+# ----------------------------------------------------------------------------------------- SAGEConv
+#   out = act(lin_l(M x) + lin_r(x)),  M = mean over the in-edges (a row without in-edges: 0);  y = dropout(out)
+#   aggregate-first (in <= out):  A = [M x | x] (saved);  [dW_l | dW_r] = gzᵀ A;  dx = Mᵀ (gz W_l) + gz W_r
+#   transform-first (in >  out):  dZ = [Mᵀ gz | gz];     [dW_l ; dW_r] = dZᵀ x;  dx = dZ [W_l ; W_r]
+# Mᵀ runs on the CSR of the reversed edges with the per-entry weight 1 / count[original target] (the kernels' src_scale).
+class SageCsr:
+    """Raw CSR of an edge_index (ops.csr_raw_from_coo) + the reversed CSR and 1/in-degree for the backward."""
+
+    def __init__(self, rowptr, col):
+        self.rowptr, self.col = rowptr, col
+        self.rowptr_t = self.col_t = self.inv_cnt = None
+
+    @staticmethod
+    def from_edge_index(edge_index, n):
+        return SageCsr(*ops.csr_raw_from_coo(edge_index, n))
+
+    def transposed(self):
+        if self.rowptr_t is None:
+            n = self.rowptr.numel() - 1
+            deg = (self.rowptr[1:] - self.rowptr[:-1]).long()
+            tgt = torch.repeat_interleave(torch.arange(n, device=self.col.device), deg)
+            self.rowptr_t, self.col_t = ops.csr_raw_from_coo(torch.stack([tgt, self.col.long()]).contiguous(), n)
+            self.inv_cnt = torch.where(deg > 0, 1.0 / deg.clamp(min=1).float(), torch.zeros((), device=deg.device)).contiguous()
+        return self.rowptr_t, self.col_t, self.inv_cnt
+
+
+def sage_weight_cat(w_l, w_r, half):
+    """[W_l | W_r] with each half zero-padded to `half` columns: the weight of the concatenated operand [M x | x]."""
+    f = w_l.shape[1]
+    pad = (0, half - f)
+    return torch.cat([torch.nn.functional.pad(w_l.detach().float(), pad), torch.nn.functional.pad(w_r.detach().float(), pad)],
+                     1).contiguous()
+
+
+class SAGEConvFn(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, w_l, b_l, w_r, csr: SageCsr, act: int, dropout_p: float = 0.0, seed: int = 0):
+        xin = _pad4(x.detach().float())
+        fin, fout = w_l.shape[1], w_l.shape[0]
+        b = b_l.detach().contiguous() if b_l is not None else None
+        ctx.csr, ctx.act, ctx.fin, ctx.fout = csr, act, fin, fout
+        ctx.p, ctx.seed = float(dropout_p), int(seed)
+        ctx.transform_first = fin > fout
+        if ctx.transform_first:
+            w = _pad4(torch.cat([w_l.detach(), w_r.detach()], 0))        # [2 out, in_p]
+            z = _linear(xin, w)
+            out = ops.spmm_mean_root(csr.rowptr, csr.col, z, fout, bias=b, act=act)
+            saved_in = xin
+        else:
+            kh = xin.shape[1]
+            w = sage_weight_cat(w_l, w_r, kh)                              # [out, 2 kh]
+            a = ops.spmm_mean_concat(csr.rowptr, csr.col, xin, kh, kh)
+            out = _linear(a, w, b, act)
+            saved_in = a
+        ctx.save_for_backward(saved_in, w, out)
+        ctx.has_bias = b_l is not None
+        if ctx.p > 0.0:
+            return ops.dropout(out, ctx.p, ctx.seed)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        saved_in, w, out = ctx.saved_tensors
+        g = g.contiguous().float()
+        gz = ops.elu_dropout_backward(g, out, ctx.act, ctx.p, ctx.seed)
+        db = gz.sum(0) if ctx.has_bias else None
+        rp_t, col_t, inv_cnt = ctx.csr.transposed()
+        fin, fout = ctx.fin, ctx.fout
+        dx = None
+        if ctx.transform_first:
+            dz = ops.spmm_mean_concat(rp_t, col_t, gz, fout, fout, src_scale=inv_cnt)  # [Mᵀ gz | gz]  [n, 2 out]
+            dw = _grad_weight(dz, saved_in)                                             # [2 out, in_p]
+            dw_l, dw_r = dw[:fout, :fin], dw[fout:, :fin]
+            if ctx.needs_input_grad[0]:
+                dx = _linear(dz, w.t().contiguous())[:, :fin]                           # dZ [W_l ; W_r]
+        else:
+            kh = w.shape[1] // 2
+            dw = _grad_weight(gz, saved_in)                                             # [out, 2 kh]
+            dw_l, dw_r = dw[:, :fin], dw[:, kh:kh + fin]
+            if ctx.needs_input_grad[0]:
+                da = _linear(gz, w.t().contiguous())                                    # [gz W_l | gz W_r]  [n, 2 kh]
+                dx = ops.spmm_mean_root(rp_t, col_t, da, kh, kh, src_scale=inv_cnt)[:, :fin]
+        return dx, dw_l.contiguous(), db, dw_r.contiguous(), None, None, None, None
+
+
+def sage_conv(x, w_l, b_l, w_r, csr: SageCsr, act: int = ops.ACT_NONE, dropout_p: float = 0.0, seed: int | None = None):
+    """dropout(act(SAGEConv(x))) (network.py:31-33 with layer_name='SAGEConv'); seed as gcn_conv."""
+    if dropout_p > 0.0 and seed is None:
+        seed = int(torch.randint(0, 2 ** 62, (1,)).item())
+    return SAGEConvFn.apply(x, w_l, b_l, w_r, csr, act, float(dropout_p), int(seed or 0))

@@ -480,6 +480,69 @@ extern "C" int fitgnn_csr_fill(int64_t n, void* ws, size_t ws_bytes, int32_t* ro
 }
 
 // =================================================================================================
+// raw CSR (drop-in SAGEConv path): the edges exactly as given — self loops kept, none added, duplicates kept
+// =================================================================================================
+namespace fitgnn {
+__global__ void csr_raw_keys_kernel(const int64_t* __restrict__ ei, int64_t E, int64_t n, uint64_t* __restrict__ keys,
+                                    int32_t* __restrict__ ctr) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= E) return;
+  const int64_t s = ei[e], d = ei[E + e];
+  if (s < 0 || s >= n || d < 0 || d >= n) {
+    atomicExch(&ctr[C_ERR], 1);
+    atomicAdd(&ctr[C_DROP], 1);
+    keys[e] = (uint64_t)n << 32;
+  } else {
+    keys[e] = ((uint64_t)d << 32) | (uint64_t)s;
+  }
+}
+}  // namespace fitgnn
+
+extern "C" int fitgnn_csr_raw_plan(const int64_t* edge_index, int64_t E, int64_t n, void* ws, size_t ws_bytes,
+                                   int64_t* host_nnz, void* stream) {
+  FG_REQUIRE(E >= 0 && n >= 0 && ws && host_nnz && (E == 0 || edge_index), FITGNN_EINVAL, "csr_raw_plan: bad arguments");
+  FG_REQUIRE(E + n < (1ll << 31) - 8192, FITGNN_ERANGE, "csr_raw_plan: E + n = %lld exceeds int32 indexing",
+             (long long)(E + n));
+  cudaStream_t st = as_stream(stream);
+  Bump b(ws, ws_bytes);
+  int32_t* ctr = b.take<int32_t>(C_N);
+  uint64_t* keys = b.take<uint64_t>((size_t)(E + n + 1));  // same layout as fitgnn_csr_plan (workspace size shared)
+  FG_REQUIRE(b.ok, FITGNN_EWS, "csr_raw_plan: workspace too small");
+  FG_CUDA(cudaMemsetAsync(ctr, 0, C_N * sizeof(int32_t), st));
+  if (E > 0) {
+    csr_raw_keys_kernel<<<nblk(E), BT, 0, st>>>(edge_index, E, n, keys, ctr);
+    FG_LAUNCH_CHECK();
+    FG_TRY(sort_u64_mask(keys, nullptr, E, field_mask((uint64_t)n, (uint64_t)n), b.here(), b.left(), st));
+  }
+  int32_t h[C_N];
+  FG_CUDA(cudaMemcpyAsync(h, ctr, sizeof(h), cudaMemcpyDeviceToHost, st));
+  FG_CUDA(cudaStreamSynchronize(st));
+  FG_REQUIRE(h[C_ERR] == 0, FITGNN_EINVAL, "csr_raw_plan: edge_index holds node ids outside [0,%lld)", (long long)n);
+  *host_nnz = E;
+  const int64_t dims[2] = {E, E};
+  FG_CUDA(cudaMemcpyAsync(ctr + 4, dims, sizeof(dims), cudaMemcpyHostToDevice, st));
+  FG_CUDA(cudaStreamSynchronize(st));
+  return FITGNN_OK;
+}
+
+extern "C" int fitgnn_csr_raw_fill(int64_t n, void* ws, size_t ws_bytes, int32_t* rowptr, int32_t* col, void* stream) {
+  FG_REQUIRE(n >= 0 && ws && rowptr, FITGNN_EINVAL, "csr_raw_fill: bad arguments");
+  cudaStream_t st = as_stream(stream);
+  Bump b(ws, ws_bytes);
+  int32_t* ctr = b.take<int32_t>(C_N);
+  int64_t dims[2];
+  FG_CUDA(cudaMemcpyAsync(dims, ctr + 4, sizeof(dims), cudaMemcpyDeviceToHost, st));
+  FG_CUDA(cudaStreamSynchronize(st));
+  const int64_t E = dims[0], nnz = dims[1];
+  uint64_t* keys = b.take<uint64_t>((size_t)(E + n + 1));
+  FG_REQUIRE(b.ok, FITGNN_EWS, "csr_raw_fill: workspace too small");
+  FG_REQUIRE(nnz == 0 || col, FITGNN_EINVAL, "csr_raw_fill: null col");
+  csr_col_kernel<<<nblk(nnz), BT, 0, st>>>(keys, nnz, col);
+  FG_LAUNCH_CHECK();
+  return segment_ptr_from_sorted(keys, nnz, 32, n, rowptr, st);
+}
+
+// =================================================================================================
 // pack builder
 // =================================================================================================
 namespace {

@@ -990,3 +990,186 @@ extern "C" int fitgnn_spmm_symnorm_grouped_f16(const int32_t* rowptr, const int3
   FG_LAUNCH_CHECK();
   return FITGNN_OK;
 }
+
+// ---------------------------------------------------------------------------------------------------------
+// SAGEConv mean aggregation (PyG SAGEConv with aggr='mean', root_weight=True):
+//   concat form: Y[i] = [ mean_{e in row r} X[src(col_e)] | X[src(r)] ]   (each half `half` columns wide, pad columns 0)
+//   root form:   Y[i] = act( mean_{e in row r} Z[src(col_e), 0:width] + Z[src(r), root_off : root_off + width] + bias )
+// r = out_rows[i].  The concat row is the A operand of ONE transform against [W_l | W_r]; the root form finishes a
+// transform-first layer whose GEMM produced Z = X·[W_l ; W_r]^T.  With skip_self the entry col == r (the single self entry
+// a pack materialises per row) is neither summed nor counted.  With src_scale the sum is weighted by src_scale[col_e] and not
+// divided (the transposed mean operator of the backward).
+// Layout as spmm_pipe_kernel: LPR lanes own a row, every lane a float4 column slice; a group reads LPR column indices at
+// once and then gathers their rows FG_SPMM_UNROLL at a time.  The sum runs in CSR order as one fmaf chain per element, then
+// ONE correctly rounded division by the count, so results do not depend on out_rows / src_index / the launch shape.
+// Rows of any length are walked in LPR-entry chunks by their own group (no hub split).
+// ---------------------------------------------------------------------------------------------------------
+namespace fitgnn {
+
+template <int NV, int LPR, bool ROOT, bool SPLIT>
+__global__ void __launch_bounds__(SPMM_THREADS, FG_SPMM_MINB)
+spmm_mean_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col, const float* __restrict__ X,
+                 int64_t ldx, int nq, int nqh, int64_t root_off, const int32_t* __restrict__ src_index,
+                 const float* __restrict__ src_scale, int skip_self, const float* __restrict__ bias, int act,
+                 const int32_t* __restrict__ out_rows, int64_t n_out, void* Y, void* Ylo, int64_t ldy) {
+  constexpr unsigned FULL = 0xffffffffu;
+  constexpr int G = 32 / LPR;
+  constexpr int U = FG_SPMM_UNROLL;
+  constexpr unsigned GMASK = LPR == 32 ? FULL : ((1u << LPR) - 1u);
+  const int lane = threadIdx.x & 31;
+  const int sub = lane & (LPR - 1);
+  const int gshift = lane & ~(LPR - 1);
+  const int64_t i = ((int64_t)blockIdx.x * SPMM_WARPS + (threadIdx.x >> 5)) * G + lane / LPR;
+  const bool live = i < n_out;
+  int r = 0, beg = 0, end = 0;  // every lane stays for the shuffles; a dead group has an empty range
+  if (live) {
+    r = out_rows ? __ldg(out_rows + i) : (int)i;
+    beg = __ldg(rowptr + r);
+    end = __ldg(rowptr + r + 1);
+  }
+  const int64_t root = live ? (src_index ? (int64_t)__ldg(src_index + r) : (int64_t)r) * ldx + root_off : 0;
+  for (int q0 = 0; q0 < nqh; q0 += LPR * NV) {
+    float4 acc[NV];
+#pragma unroll
+    for (int v = 0; v < NV; ++v) acc[v] = make_float4(0.f, 0.f, 0.f, 0.f);
+    int cnt = 0;
+    for (int e0 = beg; __any_sync(FULL, e0 < end); e0 += LPR) {
+      int c = -1;
+      if (e0 + sub < end) {
+        c = __ldg(col + e0 + sub);
+        if (skip_self && c == r) c = -1;
+      }
+      const int64_t soff = c >= 0 ? (src_index ? (int64_t)__ldg(src_index + c) : (int64_t)c) * ldx : 0;
+      const float w = (c >= 0 && src_scale) ? __ldg(src_scale + c) : 1.f;
+      const unsigned gm = (__ballot_sync(FULL, c >= 0) >> gshift) & GMASK;  // this group's live entries
+      cnt += __popc(gm);
+      const int m = __reduce_max_sync(FULL, 32 - __clz(gm));
+      for (int j = 0; j < m; j += U) {
+        float wj[U];
+        int64_t pj[U];
+        bool on[U];
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+          wj[u] = __shfl_sync(FULL, w, j + u, LPR);
+          pj[u] = __shfl_sync(FULL, soff, j + u, LPR);
+          on[u] = j + u < LPR && ((gm >> (j + u)) & 1u);
+        }
+        float4 x[U][NV];
+#pragma unroll
+        for (int u = 0; u < U; ++u)
+#pragma unroll
+          for (int v = 0; v < NV; ++v) {
+            const int q = q0 + sub + LPR * v;
+            x[u][v] = (on[u] && q < nq) ? ldg4(X + pj[u] + 4 * q) : make_float4(0.f, 0.f, 0.f, 0.f);
+          }
+#pragma unroll
+        for (int u = 0; u < U; ++u)
+          if (on[u]) {
+#pragma unroll
+            for (int v = 0; v < NV; ++v) fma4(acc[v], wj[u], x[u][v]);
+          }
+      }
+    }
+    if (!live) continue;
+    const float fc = (float)cnt;
+#pragma unroll
+    for (int v = 0; v < NV; ++v) {
+      const int q = q0 + sub + LPR * v;
+      if (q >= nqh) continue;
+      float4 o = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (q < nq) {
+        o = acc[v];
+        if (!src_scale && cnt > 0) {
+          o.x = __fdiv_rn(o.x, fc); o.y = __fdiv_rn(o.y, fc); o.z = __fdiv_rn(o.z, fc); o.w = __fdiv_rn(o.w, fc);
+        }
+      }
+      if (ROOT) {
+        const float4 z = ldg4(X + root + 4 * q);
+        o.x += z.x; o.y += z.y; o.z += z.z; o.w += z.w;
+        if (bias) {
+          const float4 b = ldg4(bias + 4 * q);
+          o.x += b.x; o.y += b.y; o.z += b.z; o.w += b.w;
+        }
+        if (act == FITGNN_ACT_ELU) {
+          o.x = elu1(o.x); o.y = elu1(o.y); o.z = elu1(o.z); o.w = elu1(o.w);
+        }
+        store_row4<SPLIT ? IO_SPLIT : IO_F32>(Y, Ylo, i * ldy + 4 * q, o);
+      } else {
+        store_row4<SPLIT ? IO_SPLIT : IO_F32>(Y, Ylo, i * ldy + 4 * q, o);
+        const float4 z = q < nq ? ldg4(X + root + 4 * q) : make_float4(0.f, 0.f, 0.f, 0.f);
+        store_row4<SPLIT ? IO_SPLIT : IO_F32>(Y, Ylo, i * ldy + 4 * (int64_t)nqh + 4 * q, z);
+      }
+    }
+  }
+}
+
+template <int NV, int LPR, bool ROOT>
+static int launch_mean(const int32_t* rowptr, const int32_t* col, const float* X, int64_t ldx, int nq, int nqh,
+                       int64_t root_off, const int32_t* src_index, const float* src_scale, int skip_self, const float* bias,
+                       int act, const int32_t* out_rows, int64_t n_out, void* Y, void* Ylo, int64_t ldy, cudaStream_t st) {
+  constexpr int G = 32 / LPR;
+  const int64_t blocks = ceil_div(n_out, (int64_t)G * SPMM_WARPS);
+  FG_REQUIRE(blocks < (1ll << 31), FITGNN_ERANGE, "spmm_mean: too many rows");
+  if (Ylo)
+    spmm_mean_kernel<NV, LPR, ROOT, true><<<(unsigned)blocks, SPMM_THREADS, 0, st>>>(
+        rowptr, col, X, ldx, nq, nqh, root_off, src_index, src_scale, skip_self, bias, act, out_rows, n_out, Y, Ylo, ldy);
+  else
+    spmm_mean_kernel<NV, LPR, ROOT, false><<<(unsigned)blocks, SPMM_THREADS, 0, st>>>(
+        rowptr, col, X, ldx, nq, nqh, root_off, src_index, src_scale, skip_self, bias, act, out_rows, n_out, Y, Ylo, ldy);
+  FG_LAUNCH_CHECK();
+  return FITGNN_OK;
+}
+
+template <bool ROOT>
+static int mean_dispatch(const int32_t* rowptr, const int32_t* col, const float* X, int64_t ldx, int nq, int nqh,
+                         int64_t root_off, const int32_t* src_index, const float* src_scale, int skip_self, const float* bias,
+                         int act, const int32_t* out_rows, int64_t n_out, void* Y, void* Ylo, int64_t ldy, void* stream) {
+  if (n_out == 0) return FITGNN_OK;
+  cudaStream_t st = as_stream(stream);
+#define FG_MEAN(NV, LPR)                                                                                                    \
+  return launch_mean<NV, LPR, ROOT>(rowptr, col, X, ldx, nq, nqh, root_off, src_index, src_scale, skip_self, bias, act,   \
+                                    out_rows, n_out, Y, Ylo, ldy, st)
+  // (float4 per lane, lanes per row) from the output half's width, as spmm_dispatch; wider rows loop over 512-column blocks
+  if (nqh <= 8) { FG_MEAN(1, 8); }
+  if (nqh <= 16) { FG_MEAN(2, 8); }
+  if (nqh <= 32) { FG_MEAN(4, 8); }
+  if (nqh <= 64) { FG_MEAN(4, 16); }
+  FG_MEAN(4, 32);
+#undef FG_MEAN
+}
+
+}  // namespace fitgnn
+
+extern "C" int fitgnn_spmm_mean_concat(const int32_t* rowptr, const int32_t* col, const float* X, int64_t ldx, int width,
+                                       int half, const int32_t* src_index, const float* src_scale, int skip_self,
+                                       const int32_t* out_rows, int64_t n_out, void* Y, void* Y_lo, int64_t ldy, void* stream) {
+  FG_REQUIRE(rowptr && col && X && Y, FITGNN_EINVAL, "spmm_mean_concat: null pointer");
+  FG_REQUIRE(n_out >= 0 && width > 0 && half >= width, FITGNN_EINVAL, "spmm_mean_concat: n_out=%lld width=%d half=%d",
+             (long long)n_out, width, half);
+  FG_REQUIRE(width % 4 == 0 && half % 4 == 0 && ldx % 4 == 0 && ldy % 4 == 0 && ldy >= 2 * (int64_t)half, FITGNN_EUNSUP,
+             "spmm_mean_concat: width (%d), half (%d), ldx (%lld), ldy (%lld) must be multiples of 4, ldy >= 2 * half", width,
+             half, (long long)ldx, (long long)ldy);
+  FG_REQUIRE(((uintptr_t)X % 16) == 0 && ((uintptr_t)Y % (Y_lo ? 8 : 16)) == 0 && ((uintptr_t)Y_lo % 8) == 0, FITGNN_EUNSUP,
+             "spmm_mean_concat: X must be 16-byte aligned, Y 16-byte (fp32) / 8-byte (planes)");
+  return mean_dispatch<false>(rowptr, col, X, ldx, width / 4, half / 4, 0, src_index, src_scale, skip_self, nullptr,
+                              FITGNN_ACT_NONE, out_rows, n_out, Y, Y_lo, ldy, stream);
+}
+
+extern "C" int fitgnn_spmm_mean_root(const int32_t* rowptr, const int32_t* col, const float* Z, int64_t ldz, int width,
+                                     int64_t root_off, const int32_t* src_index, const float* src_scale, int skip_self,
+                                     const float* bias, int act, const int32_t* out_rows, int64_t n_out, void* Y, void* Y_lo,
+                                     int64_t ldy, void* stream) {
+  FG_REQUIRE(rowptr && col && Z && Y, FITGNN_EINVAL, "spmm_mean_root: null pointer");
+  FG_REQUIRE(n_out >= 0 && width > 0 && root_off >= 0, FITGNN_EINVAL, "spmm_mean_root: n_out=%lld width=%d root_off=%lld",
+             (long long)n_out, width, (long long)root_off);
+  FG_REQUIRE(width % 4 == 0 && root_off % 4 == 0 && ldz % 4 == 0 && ldy % 4 == 0 && ldy >= width && width <= ldz &&
+                 root_off + width <= ldz,
+             FITGNN_EUNSUP, "spmm_mean_root: width (%d), root_off (%lld), ldz (%lld), ldy (%lld): multiples of 4, "
+             "root_off + width <= ldz", width, (long long)root_off, (long long)ldz, (long long)ldy);
+  FG_REQUIRE(((uintptr_t)Z % 16) == 0 && ((uintptr_t)Y % (Y_lo ? 8 : 16)) == 0 && ((uintptr_t)Y_lo % 8) == 0 &&
+                 (!bias || ((uintptr_t)bias % 16) == 0),
+             FITGNN_EUNSUP, "spmm_mean_root: Z / bias must be 16-byte aligned, Y 16-byte (fp32) / 8-byte (planes)");
+  FG_REQUIRE(act == FITGNN_ACT_NONE || act == FITGNN_ACT_ELU, FITGNN_EINVAL, "spmm_mean_root: unknown act %d", act);
+  return mean_dispatch<true>(rowptr, col, Z, ldz, width / 4, width / 4, root_off, src_index, src_scale, skip_self, bias, act,
+                             out_rows, n_out, Y, Y_lo, ldy, stream);
+}

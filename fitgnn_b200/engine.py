@@ -13,6 +13,15 @@ Schedule (SURVEY §7 ideas 2-4; all preserve the reference's arithmetic up to fp
                            regime of high coarsening ratios, e.g. the products workload) the pack is group-aligned once
                            and layers >= 1 get their propagate from the PREVIOUS transform's epilogue
                            (fitgnn_gcn_transform_aggregate): no SpMM launch and no fp32 round trip of the hidden state
+
+SAGEConv state_dicts (conv.{i}.lin_l.weight / lin_l.bias / lin_r.weight) run the classic schedule with the mean
+aggregation of spmm.cu: layer 0 aggregate-first on the operand [mean x | x] (one GEMM against [W_l | W_r]) or, F > hidden,
+transform-first Z = X·[W_l ; W_r]^T on the de-duplicated rows followed by mean + root + bias + ELU through gid; later layers
+aggregate-first; the last one on the output rows only; then the head.  The pack's CSR is used as is and its one self entry
+per row is the root, not a neighbour (skip_self).  A pack collapses the self-loop edges of its input into that single entry,
+so on a graph with self-loop edges the pack result differs from PyG's SAGEConv, which counts such an edge as a neighbour;
+the subgraphs the reference builds have none.  bf16x3 or fp32 only (the fp16 precisions run bf16x3, as for packs that are
+not eligible for the fused schedule); the fused aggregation is not built for SAGE.
 """
 from __future__ import annotations
 
@@ -26,6 +35,11 @@ _HEADS = {"identity": ops.HEAD_IDENTITY, "log_softmax": ops.HEAD_LOG_SOFTMAX, "s
 
 def conv_layers(sd):
     return len({k.split(".")[1] for k in sd if k.startswith("conv.")})
+
+
+def is_sage(sd):
+    """A SAGEConv state_dict (PyG SAGEConv keys lin_l / lin_r) rather than a GCNConv one."""
+    return "conv.0.lin_l.weight" in sd
 
 
 class PackedForward:
@@ -59,6 +73,10 @@ class PackedForward:
         self.head = _HEADS[head]
         self.with_head = with_head
         f32 = dict(dtype=torch.float32, device=dev)
+        self.sage = is_sage(state_dict)
+        if self.sage:
+            self._init_sage(state_dict, rows, fuse_aggregate, out_map, f32)
+            return
         self.W, self.b = [], []
         for i in range(self.L):
             w = state_dict[f"conv.{i}.lin.weight"].detach().to(**f32)
@@ -71,18 +89,7 @@ class PackedForward:
             self.Wl = self._prep_weight(state_dict["lt1.weight"].detach().to(**f32))
             self.bl = state_dict["lt1.bias"].detach().to(**f32).contiguous()
             self.C = state_dict["lt1.weight"].shape[0]
-        if rows == "core":
-            self.out_rows = pack.core_rows
-        elif rows == "mask":
-            self.out_rows = pack.mask_rows()
-        elif rows == "all":
-            self.out_rows = None
-        else:
-            self.out_rows = rows.to(device=dev, dtype=torch.int32).contiguous()
-        if self.out_rows is not None and self.out_rows.numel() == pack.n_rows and bool(
-                (self.out_rows.long() == torch.arange(pack.n_rows, device=dev)).all()):
-            self.out_rows = None  # identity selection (e.g. mode 'none'): skip the row indirection in the kernels
-        self.n_out = pack.n_rows if self.out_rows is None else self.out_rows.numel()
+        self._select_rows(rows)
         self.Fp = self._kpad(self.F)
         self.transform_first = self.F > self.H
         # high-degree rows are split across a CTA (found once; the pack is immutable)
@@ -182,6 +189,99 @@ class PackedForward:
             if self.out_map is not None:
                 o = self.apack.orig_row.long()
                 self._head_map = torch.where(o >= 0, self.out_map.long()[o.clamp(min=0)], o).to(torch.int32).contiguous()
+
+    def _select_rows(self, rows):
+        pack, dev = self.pack, self.pack.device
+        if rows == "core":
+            self.out_rows = pack.core_rows
+        elif rows == "mask":
+            self.out_rows = pack.mask_rows()
+        elif rows == "all":
+            self.out_rows = None
+        else:
+            self.out_rows = rows.to(device=dev, dtype=torch.int32).contiguous()
+        if self.out_rows is not None and self.out_rows.numel() == pack.n_rows and bool(
+                (self.out_rows.long() == torch.arange(pack.n_rows, device=dev)).all()):
+            self.out_rows = None  # identity selection (e.g. mode 'none'): skip the row indirection in the kernels
+        self.n_out = pack.n_rows if self.out_rows is None else self.out_rows.numel()
+
+    def _init_sage(self, sd, rows, fuse_aggregate, out_map, f32):
+        """SAGEConv weights for the classic schedule (module docstring)."""
+        from .autograd import sage_weight_cat
+        if fuse_aggregate is True:
+            raise ValueError("fuse_aggregate=True: the fused aggregation is not built for SAGEConv models")
+        self.f16_hidden = self.w_single = self.f16_classic = self.f16_layer0 = self.conv_fused = False
+        self.apack, self._blk, self._head_map = None, None, None
+        self.fused_layer0 = False
+        self.prof, self.launches, self._nnz_cache = None, 0, {}
+        w0 = sd["conv.0.lin_l.weight"]
+        self.F, self.H = w0.shape[1], w0.shape[0]
+        assert self.H % 4 == 0, "hidden width must be a multiple of 4"
+        self.Fp, self.Hp = self._kpad(self.F), self._kpad(self.H)
+        self.transform_first = self.F > self.H
+        self.W, self.b = [], []
+        for i in range(self.L):
+            wl = sd[f"conv.{i}.lin_l.weight"].detach().to(**f32)
+            wr = sd[f"conv.{i}.lin_r.weight"].detach().to(**f32)
+            if i == 0 and self.transform_first:
+                w = torch.cat([wl, wr], 0)  # [2H, F]: Z = X·[W_l ; W_r]^T
+            else:
+                w = sage_weight_cat(wl, wr, self.Fp if i == 0 else self.Hp)  # [H, 2 half]: [mean x | x]·[W_l | W_r]^T
+            self.W.append(self._prep_weight(w))
+            self.b.append(sd[f"conv.{i}.lin_l.bias"].detach().to(**f32).contiguous())
+        if self.with_head:
+            self.Wl = self._prep_weight(sd["lt1.weight"].detach().to(**f32))
+            self.bl = sd["lt1.bias"].detach().to(**f32).contiguous()
+            self.C = sd["lt1.weight"].shape[0]
+        self._select_rows(rows)
+        self.out_map = None
+        if out_map is not None:
+            assert self.with_head, "out_map needs the head"
+            self.out_map = out_map.to(device=self.pack.device, dtype=torch.int32).contiguous()
+            assert self.out_map.numel() == self.n_out
+
+    def _mean(self, name, fn, width, in_cols, out_cols, src_index, last, n_src_rows, out_elem):
+        """One mean-aggregation launch; bytes: rowptr + col, every distinct source row once (in_cols wide: the root form
+        reads both halves of Z), the output rows, gid and the row selection."""
+        p = self.pack
+        key = ("nnz", last)
+        if key not in self._nnz_cache:
+            r = self.out_rows.long() if (last and self.out_rows is not None) else None
+            self._nnz_cache[key] = p.nnz if r is None else int((p.rowptr.long()[r + 1] - p.rowptr.long()[r]).sum())
+        r_out = self.n_out if last else p.n_rows
+        nb = 4 * (r_out + 1) + 4 * self._nnz_cache[key] + 4 * n_src_rows * in_cols + out_elem * r_out * out_cols
+        nb += 4 * p.n_rows if src_index is not None else 0
+        nb += 4 * r_out if (last and self.out_rows is not None) else 0
+        self.launches += 1
+        return self._timed(name, fn, nbytes=nb, flops=self._nnz_cache[key] * width)
+
+    def _forward_sage(self, X, out, packed):
+        p = self.pack
+        bf = self.precision == ops.GEMM_BF16X3
+        X = self.pad_features(X)
+        gid0 = None if packed else p.gid
+        H, Fp, Hp = self.H, self.Fp, self.Hp
+        h = None
+        for i in range(self.L):
+            last = i == self.L - 1
+            rows = self.out_rows if last else None
+            if i == 0 and self.transform_first:
+                A = ops.split_bf16(X) if bf else X
+                if bf:
+                    self.launches += 1
+                Z = self._gemm(A, self.W[0], None, ops.ACT_NONE, N=2 * H, K=Fp, name="gemm0_unique_rows")
+                h = self._mean("mean0", lambda: ops.spmm_mean_root(p.rowptr, p.col, Z, H, H, gid0, None, True, self.b[0],
+                                                                     ops.ACT_ELU, rows),
+                               H, 2 * H, H, gid0, last, Z.shape[0], 4)
+                continue
+            src, width, half, idx = (X, Fp, Fp, gid0) if i == 0 else (h, H, Hp, None)
+            n_src = src.shape[0] if idx is not None else p.n_rows
+            A = self._mean(f"mean{i}", lambda: ops.spmm_mean_concat(p.rowptr, p.col, src, width, half, idx, None, True, rows,
+                                                                    split=bf),
+                           width, width, 2 * half, idx, last, n_src, 4)
+            to_head = bf and last and self.with_head and H % 8 == 0
+            h = self._gemm(A, self.W[i], self.b[i], ops.ACT_ELU, N=H, K=2 * half, name=f"gemm{i}", split_out=to_head)
+        return self._finish(h, out, X.device)
 
     # -- per-kernel timing for the roofline report (CUDA events on the launching stream) ---------
     def enable_profile(self, on=True):
@@ -462,10 +562,16 @@ class PackedForward:
         `out` ([n_out, C] fp32, e.g. this rank's slot of an all-gather buffer) receives the head output in place.
         `peer_ptrs` (dist.PeerGather.slot_ptrs; fused-aggregation schedule only): the head stores its rows into that slot
         of every rank's gather buffer instead (pitch pad4(C)) and nothing is returned."""
+        if self.sage and peer_ptrs is not None:
+            raise NotImplementedError("peer stores (dist.PeerGather) are built for GCNConv models only, not SAGEConv")
         assert peer_ptrs is None or self.apack is not None, "peer stores need the group-aligned schedule"
         assert self.out_map is None or (out is not None and peer_ptrs is None), "out_map needs the `out` tensor"
         p = self.pack
         assert X.is_cuda and X.dtype == torch.float32
+        if self.sage:
+            assert X.shape[0] == (p.n_rows if packed else p.n_src) and X.shape[1] in (self.F, ops.pad4(self.F), self.Fp), \
+                tuple(X.shape)
+            return self._forward_sage(X, out, packed)
         n_in = (self.apack if self.apack is not None else p).n_rows if packed else p.n_src
         assert X.shape[0] == n_in and X.shape[1] in (self.F, ops.pad4(self.F), self.Fp), tuple(X.shape)
         bf = self.precision == ops.GEMM_BF16X3
@@ -499,6 +605,11 @@ class PackedForward:
                 to_head = bf and last and self.with_head and self.H % 8 == 0
                 h = self._gemm(A, self.W[i], self.b[i], ops.ACT_ELU, N=self.H, K=width, name=f"gemm{i}",
                                split_out=to_head)
+        return self._finish(h, out, X.device)
+
+    def _finish(self, h, out, device):
+        """Head of the classic schedule on the last hidden state h (fp32, or bf16 planes from the last transform)."""
+        bf = self.precision == ops.GEMM_BF16X3
         if not self.with_head:
             return h
         if bf and not isinstance(h, tuple):
@@ -518,7 +629,7 @@ class PackedForward:
             return out
         if out is None and self.C % 4 != 0:
             # 16-byte aligned row pitch -> coalesced / TMA stores in the head epilogue; callers get the [:, :C] view
-            out = torch.empty(self.n_out, ops.pad4(self.C), dtype=torch.float32, device=X.device)
+            out = torch.empty(self.n_out, ops.pad4(self.C), dtype=torch.float32, device=device)
             view = out[:, : self.C]
         res = self._gemm(h, self.Wl, self.bl, ops.ACT_NONE, self.head, N=self.C, K=self.H, name="head", out=out)
         return res if view is None else view

@@ -16,7 +16,7 @@ from __future__ import annotations
 import torch
 
 from . import ops
-from .autograd import CsrPair, gcn_conv
+from .autograd import CsrPair, SageCsr, gcn_conv, sage_conv, sage_weight_cat
 from .engine import PackedForward
 from .pack import Pack
 
@@ -35,17 +35,18 @@ def set_precision(precision: str) -> str:
     return old
 
 
-_CSR_CACHE: dict = {}  # id(edge_index) -> (weakref to the tensor, version, n, CsrPair)
+_CSR_CACHE: dict = {}  # (kind, id(edge_index)) -> (weakref to the tensor, version, n, CsrPair | SageCsr)
 _CSR_CACHE_MAX = 64
 
 
-def _csr_for(edge_index, n):
+def _csr_for(edge_index, n, kind=CsrPair):
     """gcn_norm structure, cached per edge_index TENSOR OBJECT (PyG recomputes it on every call; cached=False).
     The entry is valid only while that very tensor is alive and unmodified: the weak reference must still resolve to
     the same object (an address or id reused by a new tensor can never alias a stale entry) and `_version` must match
-    (in-place edits invalidate)."""
+    (in-place edits invalidate).  kind: CsrPair (gcn_norm structure) or SageCsr (the edges as given); the two never share an
+    entry."""
     import weakref
-    key = id(edge_index)
+    key = (kind, id(edge_index))
     hit = _CSR_CACHE.get(key)
     if hit is not None:
         ref, version, n_hit, csr = hit
@@ -56,7 +57,7 @@ def _csr_for(edge_index, n):
             del _CSR_CACHE[k]
         if len(_CSR_CACHE) >= _CSR_CACHE_MAX:
             _CSR_CACHE.clear()
-    csr = CsrPair.from_edge_index(edge_index, n)
+    csr = kind.from_edge_index(edge_index, n)
     _CSR_CACHE[key] = (weakref.ref(edge_index), edge_index._version, n, csr)
     return csr
 
@@ -137,13 +138,72 @@ class GCNConv(torch.nn.Module):
         return f"{self.in_channels}, {self.out_channels}"
 
 
-_LAYERS = {"GCNConv": GCNConv}
+class SAGEConv(torch.nn.Module):
+    """Replacement for torch_geometric.nn.SAGEConv as `SAGEConv(in_channels, out_channels)` builds it (aggr='mean',
+    normalize=False, root_weight=True, project=False, bias=True):  out_i = lin_l(mean_{j->i} x_j) + lin_r(x_i).
+    Parameters lin_l.weight [out,in], lin_l.bias [out], lin_r.weight [out,in] (no bias).  Messages flow from
+    edge_index[0] to edge_index[1]; no self loop is added, one in edge_index is an ordinary neighbour; duplicate edges count
+    once per occurrence; a node without in-edges gets mean 0."""
+
+    _DEFAULTS = dict(aggr="mean", normalize=False, root_weight=True, project=False, bias=True)
+
+    def __init__(self, in_channels: int, out_channels: int, **kwargs):
+        super().__init__()
+        bad = sorted(k for k, v in kwargs.items() if k not in self._DEFAULTS or v != self._DEFAULTS[k])
+        if bad:
+            raise TypeError(f"unsupported SAGEConv options: {bad}")
+        self.in_channels, self.out_channels = in_channels, out_channels
+        self.lin_l = torch.nn.Linear(in_channels, out_channels, bias=True)
+        self.lin_r = torch.nn.Linear(in_channels, out_channels, bias=False)
+        self.reset_parameters()
+
+    def reset_parameters(self):
+        self.lin_l.reset_parameters()  # PyG Linear: kaiming_uniform(a=sqrt(5)) weight, uniform bias — torch.nn.Linear's
+        self.lin_r.reset_parameters()
+
+    def forward(self, x, edge_index, act: int = ops.ACT_NONE, dropout_p: float = 0.0):
+        """act / dropout_p: the F.elu / F.dropout that follow the conv in every reference model, fused as in GCNConv."""
+        _require_cuda(x)
+        if self.out_channels % 4 != 0:
+            raise RuntimeError("fitgnn_b200.SAGEConv needs out_channels % 4 == 0")
+        n = x.shape[0]
+        csr = _csr_for(edge_index, n, SageCsr)
+        wl, bl, wr = self.lin_l.weight, self.lin_l.bias, self.lin_r.weight
+        if torch.is_grad_enabled() and (x.requires_grad or wl.requires_grad or bl.requires_grad or wr.requires_grad):
+            return sage_conv(x, wl, bl, wr, csr, act, dropout_p)
+        if dropout_p > 0.0:
+            y = self.forward(x, edge_index, act)
+            return ops.dropout(y, dropout_p, int(torch.randint(0, 2 ** 62, (1,)).item()))
+        b = bl.detach().contiguous()
+        align = 8 if _PRECISION == "bf16x3" else 4
+        xp = _as_f32_padded(x.detach(), align)
+        if self.in_channels > self.out_channels:  # Z = x [W_l ; W_r]^T on the wide rows, then mean + root + bias + act
+            w = torch.cat([wl.detach(), wr.detach()], 0)
+            if _PRECISION == "bf16x3":
+                z = ops.linear_tc(xp, w)
+            else:
+                z = ops.gemm_bias_act(xp, _pad_weight(w), None, ops.ACT_NONE, K=xp.shape[1])
+            return ops.spmm_mean_root(csr.rowptr, csr.col, z, self.out_channels, bias=b, act=act)
+        # aggregate-first: [mean x | x] as ONE operand, one GEMM against [W_l | W_r]
+        kh = xp.shape[1]
+        w = sage_weight_cat(wl, wr, kh)
+        if _PRECISION == "bf16x3":
+            a = ops.spmm_mean_concat(csr.rowptr, csr.col, xp, kh, kh, split=True)
+            return ops.linear_tc(None, w, b, act, x_planes=a)
+        a = ops.spmm_mean_concat(csr.rowptr, csr.col, xp, kh, kh)
+        return ops.gemm_bias_act(a, w, b, act, K=2 * kh)
+
+    def extra_repr(self):
+        return f"{self.in_channels}, {self.out_channels}, aggr=mean"
+
+
+_LAYERS = {"GCNConv": GCNConv, "SAGEConv": SAGEConv}
 
 
 def _layer_class(args):
     name = getattr(args, "layer_name", "GCNConv")
     if name not in _LAYERS:
-        raise NotImplementedError(f"layer_name={name!r}: only GCNConv is on the B200 hot path (SURVEY §2 row 15)")
+        raise NotImplementedError(f"layer_name={name!r}: only {sorted(_LAYERS)} are on the B200 hot path (SURVEY §2 row 15)")
     return _LAYERS[name]
 
 
@@ -287,31 +347,33 @@ class Regress_graph_gs(_GraphGs):
         return self._forward_gs(set_gs, batch_tensor, ops.POOL_MEAN, ops.HEAD_IDENTITY)
 
 
-def _ns(num_features, hidden, num_layers, num_classes):
+def _ns(num_features, hidden, num_layers, num_classes, layer_name="GCNConv"):
     import argparse
     return argparse.Namespace(num_features=num_features, hidden=hidden, num_layers1=num_layers,
-                              num_classes=num_classes, layer_name="GCNConv")
+                              num_classes=num_classes, layer_name=layer_name)
 
 
 class Net1(Classify_node):
-    """inference.py:72-93 `Net1(num_features, hidden, num_layers, num_classes)` — same state_dict keys."""
+    """inference.py:72-93 `Net1(num_features, hidden, num_layers, num_classes)` — same state_dict keys.  layer_name: the
+    conv class, as args.layer_name of the network.py models."""
 
-    def __init__(self, num_features, hidden, num_layers, num_classes):
-        super().__init__(_ns(num_features, hidden, num_layers, num_classes))
+    def __init__(self, num_features, hidden, num_layers, num_classes, layer_name="GCNConv"):
+        super().__init__(_ns(num_features, hidden, num_layers, num_classes, layer_name))
 
 
 class Net2(Regress_node):
     """inference.py:95-116 `Net2(num_features, hidden, num_layers)`."""
 
-    def __init__(self, num_features, hidden, num_layers, num_classes=1):
-        super().__init__(_ns(num_features, hidden, num_layers, 1))
+    def __init__(self, num_features, hidden, num_layers, num_classes=1, layer_name="GCNConv"):
+        super().__init__(_ns(num_features, hidden, num_layers, 1, layer_name))
 
 
 def install():
     """Route the reference's layer lookup to this module: after `fitgnn_b200.nn.install()`,
-    `getattr(torch_geometric.nn, 'GCNConv')` (network.py:13) and `from torch_geometric.nn import GCNConv`
-    (network.py:5, inference.py) resolve to the B200 operator.  Call before importing network.py."""
+    `getattr(torch_geometric.nn, 'GCNConv')` / `'SAGEConv'` (network.py:13) and `from torch_geometric.nn import GCNConv`
+    (network.py:5, inference.py) resolve to the B200 operators.  Call before importing network.py."""
     import importlib
     pyg_nn = importlib.import_module("torch_geometric.nn")
     pyg_nn.GCNConv = GCNConv
+    pyg_nn.SAGEConv = SAGEConv
     return pyg_nn

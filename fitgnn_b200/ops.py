@@ -58,6 +58,62 @@ def csr_from_coo(edge_index, n):
     return rowptr, col, dinv
 
 
+def csr_raw_from_coo(edge_index, n):
+    """CSR of the edges exactly as given (drop-in SAGEConv): (rowptr, col), rows = targets, self loops and duplicate
+    edges kept as ordinary entries, none added; columns ascending inside a row."""
+    assert edge_index.dtype == torch.int64 and edge_index.dim() == 2 and edge_index.shape[0] == 2
+    ei = edge_index.contiguous()
+    E = ei.shape[1]
+    ws = _ws(lib().fitgnn_csr_workspace_bytes(E, n), ei.device)
+    nnz = C.c_int64(0)
+    check(lib().fitgnn_csr_raw_plan(ptr(ei), E, n, ptr(ws), ws.numel(), C.byref(nnz), stream_ptr()))
+    rowptr = torch.empty(n + 1, dtype=torch.int32, device=ei.device)
+    col = torch.empty(max(nnz.value, 1), dtype=torch.int32, device=ei.device)[: nnz.value]
+    check(lib().fitgnn_csr_raw_fill(n, ptr(ws), ws.numel(), ptr(rowptr), ptr(col), stream_ptr()))
+    return rowptr, col
+
+
+def _mean_out(n_out, ncols, split, out, device):
+    if split:
+        if out is None:
+            out = (torch.empty(n_out, ncols, dtype=torch.bfloat16, device=device),
+                   torch.empty(n_out, ncols, dtype=torch.bfloat16, device=device))
+        return out, out[0], out[1], out[0].stride(0)
+    if out is None:
+        out = torch.empty(n_out, ncols, dtype=torch.float32, device=device)
+    return out, out, None, out.stride(0)
+
+
+def spmm_mean_concat(rowptr, col, X, width=None, half=None, src_index=None, src_scale=None, skip_self=False, out_rows=None,
+                     out=None, split=False):
+    """SAGEConv operand: Y[i] = [mean_j X[src(j)] | X[src(r_i)]], halves `half` columns apart (default width), pad columns
+    zero (fitgnn_spmm_mean_concat).  split=True returns bf16 (hi, lo) planes [n_out, 2*half] for the tensor-core GEMM.
+    skip_self: the entry col == row is not a neighbour (pack CSRs); src_scale: weighted sum instead of the mean."""
+    assert X.dtype == torch.float32 and X.dim() == 2
+    width = X.shape[1] if width is None else width
+    half = width if half is None else half
+    n_out = out_rows.numel() if out_rows is not None else rowptr.numel() - 1
+    out, y, ylo, ldy = _mean_out(n_out, 2 * half, split, out, X.device)
+    check(lib().fitgnn_spmm_mean_concat(ptr(rowptr), ptr(col), ptr(X), X.stride(0), width, half, ptr(src_index),
+                                        ptr(src_scale), int(bool(skip_self)), ptr(out_rows), n_out, ptr(y), ptr(ylo), ldy,
+                                        stream_ptr()))
+    return out
+
+
+def spmm_mean_root(rowptr, col, Z, width, root_off=None, src_index=None, src_scale=None, skip_self=False, bias=None,
+                   act=ACT_NONE, out_rows=None, out=None, split=False):
+    """Transform-first SAGEConv: Y[i] = act(mean_j Z[src(j), :width] + Z[src(r_i), root_off:root_off+width] + bias) with
+    Z = X·[W_l ; W_r]^T (root_off defaults to width) (fitgnn_spmm_mean_root)."""
+    assert Z.dtype == torch.float32 and Z.dim() == 2
+    root_off = width if root_off is None else root_off
+    n_out = out_rows.numel() if out_rows is not None else rowptr.numel() - 1
+    out, y, ylo, ldy = _mean_out(n_out, width, split, out, Z.device)
+    check(lib().fitgnn_spmm_mean_root(ptr(rowptr), ptr(col), ptr(Z), Z.stride(0), width, root_off, ptr(src_index),
+                                      ptr(src_scale), int(bool(skip_self)), ptr(bias), act, ptr(out_rows), n_out, ptr(y),
+                                      ptr(ylo), ldy, stream_ptr()))
+    return out
+
+
 def spmm_symnorm(rowptr, col, dinv, X, width=None, src_index=None, bias=None, act=ACT_NONE, out_rows=None,
                  out=None, split=False, hubs=None):
     """Y = act(Â·X[src_index] + bias) on the rows `out_rows` (all rows when None).
@@ -340,6 +396,8 @@ def gcn_forward(pack, X, state_dict, head=HEAD_LOG_SOFTMAX, precision=GEMM_BF16X
     core rows, classic schedule.  pack: fitgnn_b200.pack.Pack; X: [n_src, F] fp32 feature table; state_dict: the
     reference's keys (conv.{i}.lin.weight, conv.{i}.bias, lt1.weight, lt1.bias).  Returns [n_core, C]."""
     from ._lib import WeightsStruct
+    if "conv.0.lin_l.weight" in state_dict:
+        raise NotImplementedError("fitgnn_gcn_forward runs GCNConv models only; run a SAGEConv model with PackedForward")
     dev = X.device
     L = len({k.split(".")[1] for k in state_dict if k.startswith("conv.")})
     f32 = dict(dtype=torch.float32, device=dev)

@@ -17,7 +17,7 @@ from __future__ import annotations
 import torch
 
 from . import ops
-from .engine import PackedForward
+from .engine import PackedForward, is_sage
 from .infer import select_subgraphs
 from .pack import Pack, PackStream
 
@@ -27,6 +27,9 @@ class StreamedForward:
 
     def __init__(self, packs, state_dict, head="log_softmax", precision="bf16x3", hybrid="auto", small_rows=32,
                  align_policy="degree", min_small_fraction=0.05):
+        if is_sage(state_dict):
+            raise NotImplementedError("StreamedForward runs GCNConv models only; run a SAGEConv model per pack with "
+                                      "PackedForward")
         if isinstance(packs, Pack):
             packs = PackStream([packs], [0, packs.n_sub], packs.mode, packs.n_nodes, packs.n_src)
         self.stream = packs

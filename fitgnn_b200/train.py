@@ -6,7 +6,7 @@ from __future__ import annotations
 
 import torch
 
-from .autograd import CsrPair
+from .autograd import CsrPair, SageCsr
 from .pack import Pack
 
 
@@ -14,15 +14,30 @@ def pack_csr(pack: Pack) -> CsrPair:
     return CsrPair(pack.rowptr, pack.col, pack.dinv)
 
 
-def forward_on_pack(model, pack: Pack, X, csr: CsrPair | None = None):
-    """Differentiable forward of a node model (fitgnn_b200.nn.Classify_node / Regress_node) over every row of the pack;
-    X is the de-duplicated feature table ([N (+k), F]).  Returns [n_rows, C] with grad_fn."""
+def pack_sage_csr(pack: Pack) -> SageCsr:
+    """The pack's CSR without its self entries (the SAGEConv root, not a neighbour; as PackedForward's skip_self).  Built
+    with a sort: pass it to forward_on_pack / train_step_Gs as `csr` to reuse it across steps."""
+    rp = pack.rowptr.long()
+    row = torch.repeat_interleave(torch.arange(pack.n_rows, device=rp.device), rp[1:] - rp[:-1])
+    col = pack.col.long()
+    keep = col != row
+    return SageCsr.from_edge_index(torch.stack([col[keep], row[keep]]).contiguous(), pack.n_rows)
+
+
+def forward_on_pack(model, pack: Pack, X, csr: CsrPair | SageCsr | None = None):
+    """Differentiable forward of a node model (fitgnn_b200.nn.Classify_node / Regress_node, GCNConv or SAGEConv layers)
+    over every row of the pack; X is the de-duplicated feature table ([N (+k), F]).  Returns [n_rows, C] with grad_fn."""
     from . import ops
-    from .autograd import gcn_conv
-    csr = csr or pack_csr(pack)
+    from .autograd import gcn_conv, sage_conv
+    sage = hasattr(model.conv[0], "lin_l")
+    csr = csr or (pack_sage_csr(pack) if sage else pack_csr(pack))
     x = X[pack.gid.long()]
     for i in range(model.num_layers):  # conv -> ELU -> dropout (network.py:31-33, p = 0.5 in train mode), one fused operator
-        x = gcn_conv(x, model.conv[i].lin.weight, model.conv[i].bias, csr, ops.ACT_ELU, 0.5 if model.training else 0.0)
+        c, p = model.conv[i], 0.5 if model.training else 0.0
+        if sage:
+            x = sage_conv(x, c.lin_l.weight, c.lin_l.bias, c.lin_r.weight, csr, ops.ACT_ELU, p)
+        else:
+            x = gcn_conv(x, c.lin.weight, c.bias, csr, ops.ACT_ELU, p)
     y = model.lt1(x)
     return torch.nn.functional.log_softmax(y, dim=1) if model._head == "log_softmax" else y
 

@@ -113,6 +113,13 @@ int fitgnn_csr_plan(const int64_t* edge_index, int64_t E, int64_t n, void* ws, s
                     int64_t* host_nnz, void* stream);
 int fitgnn_csr_fill(int64_t n, void* ws, size_t ws_bytes, int32_t* rowptr /*[n+1]*/,
                     int32_t* col /*[nnz]*/, float* dinv /*[n]*/, void* stream);
+/* Raw per-call CSR (drop-in SAGEConv path): the edges exactly as given — self loops kept, none added, duplicates kept
+ * (each occurrence is one entry).  Same workspace as fitgnn_csr_plan (fitgnn_csr_workspace_bytes); *host_nnz = E.  Rows are
+ * targets, entries in ascending column order inside a row.  No dinv. */
+int fitgnn_csr_raw_plan(const int64_t* edge_index, int64_t E, int64_t n, void* ws, size_t ws_bytes,
+                        int64_t* host_nnz, void* stream);
+int fitgnn_csr_raw_fill(int64_t n, void* ws, size_t ws_bytes, int32_t* rowptr /*[n+1]*/, int32_t* col /*[nnz]*/,
+                        void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Pack builder.  Replaces coarsening_classification / coarsening_regression's per-cluster
@@ -145,6 +152,25 @@ int fitgnn_spmm_symnorm(const int32_t* rowptr, const int32_t* col, const float* 
                         const float* X, int64_t ldx, int width, const int32_t* src_index,
                         const float* bias, int act, const int32_t* out_rows, int64_t n_out,
                         void* Y, void* Y_lo, int64_t ldy, void* stream);
+/* Mean aggregation of SAGEConv (PyG SAGEConv, aggr='mean', root_weight=True):  out_i = lin_l(mean_j x_j) + lin_r(x_i).
+ * r_i = out_rows[i] (or i), src(c) = src_index[c] (or c).  skip_self != 0: the entry col == r_i (the one self entry of a
+ * pack row) is neither summed nor counted; otherwise every entry is a neighbour.  A row without neighbours has mean 0.
+ * The sum runs in CSR order (one fmaf chain per element) and is divided by the neighbour count (correctly rounded), so the
+ * result is independent of out_rows / src_index.  src_scale (device, indexed by column, may be NULL): the sum is weighted by
+ * src_scale[col_e] and NOT divided — with the reversed CSR and src_scale = 1/count this is the transposed mean operator.
+ * Y as fitgnn_spmm_symnorm: fp32, or bf16 hi/lo planes when Y_lo != NULL.
+ * concat (aggregate-first):  Y[i] = [ mean X[src(col_e), 0:width] | X[src(r_i), 0:width] ], the second half starting at
+ *   column `half` (>= width); columns [width, half) and [half + width, 2*half) are written as zeros.  This is the A operand
+ *   of ONE transform against [W_l | W_r] (K = 2*half), with lin_l.bias and the activation in its epilogue.
+ * root (transform-first, after Z = X·[W_l ; W_r]^T):
+ *   Y[i] = act( mean Z[src(col_e), 0:width] + Z[src(r_i), root_off : root_off + width] + bias ). */
+int fitgnn_spmm_mean_concat(const int32_t* rowptr, const int32_t* col, const float* X, int64_t ldx, int width, int half,
+                            const int32_t* src_index, const float* src_scale, int skip_self, const int32_t* out_rows,
+                            int64_t n_out, void* Y, void* Y_lo, int64_t ldy, void* stream);
+int fitgnn_spmm_mean_root(const int32_t* rowptr, const int32_t* col, const float* Z, int64_t ldz, int width,
+                          int64_t root_off, const int32_t* src_index, const float* src_scale, int skip_self,
+                          const float* bias, int act, const int32_t* out_rows, int64_t n_out, void* Y, void* Y_lo,
+                          int64_t ldy, void* stream);
 /* The same aggregation (no bias / activation, every row an output row) for a GROUP-ALIGNED pack
  * (fitgnn_pack_align_*): every CSR entry of a row lies in the row's own group of `group` = 32 rows, so one warp stages
  * the group's source rows in shared memory once and HBM sees every byte once.  width <= 128.  Results are bit-identical
