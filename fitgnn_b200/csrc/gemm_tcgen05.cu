@@ -830,7 +830,8 @@ gemm_bf16x3_kernel(const GatherArgs ga, const EpiArgs ea, const __grid_constant_
         exchanged = true;
       };
       if (head != FITGNN_HEAD_IDENTITY && !FAST_HEAD && col_group == 0) {
-        // pass 1: online max / sum of exp over the row (the whole row lives in this tile: N <= BLOCK_N)
+        // pass 1: online max / sum of exp over the row (the whole row lives in this tile: N <= BLOCK_N).  The logits are
+        // formed exactly as pass 2 forms them (row scale included), so the statistics belong to the values they normalise.
         for (int c0 = 0; c0 < BLOCK_N; c0 += 16) {
           float v[16];
           tmem_ld16(taddr + c0, v);
@@ -838,7 +839,8 @@ gemm_bf16x3_kernel(const GatherArgs ga, const EpiArgs ea, const __grid_constant_
           for (int j = 0; j < 16; ++j) {
             const int n = n0 + c0 + j;
             if (n < N) {
-              float x = v[j] + (bias ? __ldg(bias + n) : 0.f);
+              const float b = bias ? __ldg(bias + n) : 0.f;
+              float x = ea.row_scale ? fmaf(v[j], rs, b) : v[j] + b;
               if (act == FITGNN_ACT_ELU) x = elu1(x);
               const float nm = fmaxf(row_max, x);
               row_sum = row_sum * __expf(row_max - nm) + __expf(x - nm);
@@ -984,6 +986,14 @@ gemm_bf16x3_kernel(const GatherArgs ga, const EpiArgs ea, const __grid_constant_
           // (bulk async-groups belong to a thread: elect_one picks the same lane every time)
           if (elect_one()) bulk_wait_read<0>();  // the store(s) that last read this buffer have finished reading
           __syncwarp();
+          // the TMA unit clips a row at the 16-byte boundary after column N, not at N: the columns up to it are stored too.
+          // Without a head they hold zeros already (zero-filled W rows, no bias past N, act(0) = 0); a head's normalisation
+          // would leave garbage there, so they are zeroed (the gather kernel never carries a head)
+          if (!GATHER && head != FITGNN_HEAD_IDENTITY && n0 + c0 + 32 > N) {
+#pragma unroll
+            for (int j = 0; j < 32; ++j)
+              if (n0 + c0 + j >= N) v[j] = 0.f;
+          }
           if (tma_store == 3) {  // ONE fp16 plane (64-byte rows, the bf16 planes' swizzle)
 #pragma unroll
             for (int j = 0; j < 4; ++j) {

@@ -7,7 +7,8 @@ inference.py:72-116), computing on the sm_100a kernels of libfitgnn_b200.so.
 `__call__(x[n,in] fp32, edge_index[2,E] int64) -> [n,out]`.
 
 Autograd: when gradients are enabled and a parameter (or x) requires grad, the conv runs through
-`fitgnn_b200.autograd.GCNConvFn`, whose backward uses the same kernels (SpMM with the reversed CSR, fp32 GEMMs), so
+`fitgnn_b200.autograd.GCNConvFn`, whose backward uses the same kernels (SpMM with the reversed CSR; the dX = gz·W and
+dW = gzᵀ·x products on the bf16x3 tensor cores, or on the exact-fp32 GEMM after `set_precision("fp32")`), so
 the reference's training loops (run.py:26-37, :177-215) work unchanged; `.train()` mode applies F.dropout like
 network.py:33.  Under torch.no_grad() the lean inference path is taken.  CUDA tensors only — there is no CPU path.
 """
@@ -22,7 +23,8 @@ from .pack import Pack
 
 # Arithmetic of the dense transforms on the inference (no-grad) path of the drop-in classes: 'bf16x3' = tcgen05 tensor
 # cores on a bf16 hi/lo split of both operands with fp32 accumulation (default), 'fp32' = exact-fp32 CUDA-core GEMM
-# (explicit opt-in: the numerics anchor).  The autograd path (training) uses the fp32 kernels.
+# (explicit opt-in: the numerics anchor).  The autograd path (training) follows the same setting: its forward GEMMs and the
+# dX / dW products of the backward (fitgnn_gemm_tn) run on the bf16x3 tensor cores unless 'fp32' is selected.
 _PRECISION = "bf16x3"
 
 

@@ -236,7 +236,12 @@ int fitgnn_spmm_symnorm_devhub(const int32_t* rowptr, const int32_t* col, const 
  *   Y[M,N] = act( A[M,K] · W[N,K]^T + bias[N] ),  W laid out as lin.weight ([out,in] row-major).
  * FITGNN_GEMM_FP32: A, W fp32.   FITGNN_GEMM_BF16X3: A_hi/A_lo and W_hi/W_lo are bf16 planes
  * (see fitgnn_split_bf16); K-extent padded to a multiple of 8 with zeros by the caller.
- * head != IDENTITY applies a row-wise (log-)softmax over the N outputs (N <= 256), after act.
+ * head != IDENTITY applies a row-wise (log-)softmax over the N outputs (N <= 256 for BF16X3, any N for FP32), after act.
+ * Only rows [0, M) of Y are written, and of them columns [0, N) plus, with BF16X3 when Y (and Y_lo) are 16-byte aligned
+ * with a pitch of a multiple of 16 bytes (the TMA-store path), zeros up to the next 16-byte boundary: [N, pad4(N)) of an
+ * fp32 output, [N, pad8(N)) of both split planes (which makes them the zero K-padding of the next product's operand).
+ * Every other pitch column keeps its contents.  The operands are read only in their first K columns and (W) first N
+ * rows; the pitch beyond them may hold anything.
  * ---------------------------------------------------------------------------------------- */
 int fitgnn_gemm_bias_act(int precision, const void* A, const void* A_lo, int64_t lda,
                          const void* W, const void* W_lo, int64_t ldw, const float* bias,
@@ -304,7 +309,7 @@ int fitgnn_gcn_transform_aggregate(const void* A_hi, const void* A_lo, int64_t l
                                    int N, int act, const uint64_t* agg_desc, const float* dinv,
                                    int defer_row_scale, void* Y, void* Y_lo, int64_t ldy, void* stream);
 /* fitgnn_gemm_bias_act_split with a per-row factor:  Y = head(act(row_scale[m] * (A·W^T)[m,:] + bias)).
- * row_scale may be NULL (= 1); non-NULL needs FITGNN_GEMM_BF16X3. */
+ * row_scale may be NULL (= 1); non-NULL needs FITGNN_GEMM_BF16X3.  A head normalises the scaled logits. */
 int fitgnn_gemm_rowscale_bias_act_split(int precision, const void* A, const void* A_lo, int64_t lda,
                                         const void* W, const void* W_lo, int64_t ldw,
                                         const float* row_scale, const float* bias, int64_t M, int K,
