@@ -85,6 +85,12 @@ SIGNATURES = {
     "fitgnn_split_f16": (c_i32, [c_void, c_i64, c_i64, c_i32, c_void, c_void, c_i64, c_void]),
     "fitgnn_gemm_f16": (c_i32, [c_void, c_i64, c_void, c_void, c_i64, c_void, c_void, c_i64, c_i32, c_i32, c_i32, c_i32, c_void,
                                 c_i64, c_i32, c_void, c_void]),
+    "fitgnn_spmm_mean_f16": (c_i32, [c_void, c_void, c_void, c_i64, c_i32, c_i32, c_void, c_i32, c_i32, c_void, c_i64, c_void,
+                                     c_i64, c_void]),
+    "fitgnn_spmm_mean_root_f16": (c_i32, [c_void, c_void, c_void, c_i64, c_i32, c_i64, c_void, c_i32, c_void, c_i32, c_void,
+                                          c_i64, c_void, c_i64, c_void]),
+    "fitgnn_gemm_f16_2seg": (c_i32, [c_void, c_i64, c_i32, c_i32, c_void, c_i64, c_void, c_void, c_i64, c_void, c_i64, c_i32,
+                                     c_i32, c_i32, c_void, c_i64, c_i32, c_void]),
     "fitgnn_gemm_f16_head_rows_peers": (c_i32, [c_void, c_i64, c_void, c_void, c_i64, c_void, c_i64, c_i32, c_i32, c_i32, c_i32,
                                                 c_void, C.POINTER(c_void), c_i32, c_i64, c_void]),
     "fitgnn_gcn_transform_aggregate_f16": (c_i32, [c_i32, c_void, c_void, c_i64, c_void, c_void, c_i64, c_void, c_i64, c_i32,

@@ -61,7 +61,8 @@ int gemm_bf16x3(const void* A_hi, const void* A_lo, int64_t lda, const void* W_h
                 const float* bias, int64_t M, int K, int N, int act, int head, float* Y, void* Y_lo, int64_t ldy,
                 const uint64_t* agg_desc, const float* agg_dinv, const int32_t* row_map, float* const* peers, int n_peers,
                 const float* row_scale, int agg_defer_scale, cudaStream_t st, int64_t m_batch_rows = 0, int w_batch_rows = 0,
-                int64_t w_rows_total = 0, int in_f16 = 0, int out_f16 = 0, int agg_pre = 0);
+                int64_t w_rows_total = 0, int in_f16 = 0, int out_f16 = 0, int agg_pre = 0,
+                int a_seg_k0 = 0, int a0_cols = 0, const void* A1 = nullptr, int64_t lda1 = 0);
 
 int gcn_layer_fused(const int32_t* rowptr, const int32_t* col, const float* dinv, const float* X, int64_t ldx, int width,
                     const int32_t* src_index, const int32_t* out_rows, int64_t M, const void* W_hi, const void* W_lo,
@@ -217,6 +218,23 @@ extern "C" int fitgnn_gemm_f16(const void* A, int64_t lda, const void* W_hi, con
   if (M == 0) return FITGNN_OK;
   return gemm_bf16x3(A, nullptr, lda, W_hi, W_lo, ldw, bias, M, K, N, act, head, static_cast<float*>(Y), nullptr, ldy, nullptr,
                      nullptr, row_map, nullptr, 0, row_scale, 0, as_stream(stream), 0, 0, 0, 1, out_f16 ? 1 : 0);
+}
+
+extern "C" int fitgnn_gemm_f16_2seg(const void* A0, int64_t lda0, int a0_cols, int K0, const void* A1, int64_t lda1,
+                                    const void* W_hi, const void* W_lo, int64_t ldw, const float* bias, int64_t M, int K, int N,
+                                    int act, void* Y, int64_t ldy, int out_f16, void* stream) {
+  FG_REQUIRE(A0 && A1 && W_hi && Y && M >= 0 && K > 0 && N > 0, FITGNN_EINVAL,
+             "gemm_f16_2seg: bad arguments (M=%lld K=%d N=%d)", (long long)M, K, N);
+  FG_REQUIRE(K0 > 0 && K0 % 64 == 0 && K > K0, FITGNN_EUNSUP,
+             "gemm_f16_2seg: K0 (%d) must be a positive multiple of 64 (the k-block) and below K (%d)", K0, K);
+  FG_REQUIRE(a0_cols > 0 && a0_cols <= K0, FITGNN_EINVAL, "gemm_f16_2seg: A0 has %d columns, segment 0 is %d wide", a0_cols, K0);
+  FG_REQUIRE(lda0 >= a0_cols && lda1 >= K - K0 && ldw >= K && ldy >= N, FITGNN_EINVAL,
+             "gemm_f16_2seg: leading dimension smaller than the extent");
+  FG_REQUIRE(act == FITGNN_ACT_NONE || act == FITGNN_ACT_ELU, FITGNN_EINVAL, "gemm_f16_2seg: unknown act %d", act);
+  if (M == 0) return FITGNN_OK;
+  return gemm_bf16x3(A0, nullptr, lda0, W_hi, W_lo, ldw, bias, M, K, N, act, FITGNN_HEAD_IDENTITY, static_cast<float*>(Y), nullptr,
+                     ldy, nullptr, nullptr, nullptr, nullptr, 0, nullptr, 0, as_stream(stream), 0, 0, 0, 1, out_f16 ? 1 : 0, 0,
+                     K0, a0_cols, A1, lda1);
 }
 
 extern "C" int fitgnn_gcn_transform_aggregate_f16(int in_f16, const void* A_hi, const void* A_lo, int64_t lda, const void* W_hi,

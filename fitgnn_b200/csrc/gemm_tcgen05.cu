@@ -91,6 +91,9 @@ struct EpiArgs {
   int w_planes;
   int l2_prefetch;  // producer: prefetch the next m-block's A rows into L2 (tuning switch gemm_prefetch, default off)
   int debug;        // measurement switches (tuning gemm_debug, default 0): bit 0 = the epilogue skips its TMA stores
+  // a_seg_kb > 0 (single-plane A only, fitgnn_gemm_f16_2seg): the A operand is two planes side by side in K — k-blocks
+  // [0, a_seg_kb) come from map_a_hi, the rest from map_a_lo at k-offset (kb - a_seg_kb) * BLOCK_K.  Only the producer knows.
+  int a_seg_kb;
 };
 constexpr int EPI_WARP0 = 2;
 constexpr int ACC_STAGES = 2;
@@ -486,9 +489,13 @@ gemm_bf16x3_kernel(const GatherArgs ga, const EpiArgs ea, const __grid_constant_
         }
         prev_mb = w.mb;
         for (int kb = 0; kb < k_blocks; ++kb) {
+          // the A plane of this k-block and the k-coordinate inside it (two-segment A: see EpiArgs::a_seg_kb)
+          const bool seg1 = ea.a_seg_kb > 0 && kb >= ea.a_seg_kb;
+          const CUtensorMap* map_a = seg1 ? &map_a_lo : &map_a_hi;
+          const int ka = (seg1 ? kb - ea.a_seg_kb : kb) * BLOCK_K;
           if (pf_m0 >= 0 && ea.l2_prefetch) {
             if (elect_one()) {
-              tma_prefetch_2d(&map_a_hi, kb * BLOCK_K, pf_m0);
+              tma_prefetch_2d(map_a, ka, pf_m0);
               if (!a_single) tma_prefetch_2d(&map_a_lo, kb * BLOCK_K, pf_m0);
             }
             __syncwarp();
@@ -502,7 +509,7 @@ gemm_bf16x3_kernel(const GatherArgs ga, const EpiArgs ea, const __grid_constant_
               // both CTAs' bytes are counted on the LEADER's full barrier (its MMA thread consumes both halves)
               const uint32_t lbar = mapa_rank(full_bar(stage), 0);
               if (leader) mbar_arrive_expect_tx(full_bar(stage), 2 * tx_bytes);
-              tma_load_2d_pair(dst, &map_a_hi, lbar, kb * BLOCK_K, m0);
+              tma_load_2d_pair(dst, map_a, lbar, ka, m0);
               if (!a_single) tma_load_2d_pair(dst + A_PLANE_BYTES, &map_a_lo, lbar, kb * BLOCK_K, m0);
               if (!w_stationary) {
                 tma_load_2d_pair(dst + a_bytes, &map_w_hi, lbar, kb * BLOCK_K, n0 + (int)cta_rank * B_ROWS);
@@ -511,7 +518,7 @@ gemm_bf16x3_kernel(const GatherArgs ga, const EpiArgs ea, const __grid_constant_
               }
             } else {
               mbar_arrive_expect_tx(full_bar(stage), tx_bytes);
-              tma_load_2d(dst, &map_a_hi, full_bar(stage), kb * BLOCK_K, m0);
+              tma_load_2d(dst, map_a, full_bar(stage), ka, m0);
               if (!a_single) tma_load_2d(dst + A_PLANE_BYTES, &map_a_lo, full_bar(stage), kb * BLOCK_K, m0);
               if (!w_stationary) {
                 tma_load_2d(dst + a_bytes, &map_w_hi, full_bar(stage), kb * BLOCK_K, n0);
@@ -1287,8 +1294,12 @@ int gemm_bf16x3(const void* A_hi, const void* A_lo, int64_t lda, const void* W_h
                 const float* bias, int64_t M, int K, int N, int act, int head, float* Y, void* Y_lo, int64_t ldy,
                 const uint64_t* agg_desc, const float* agg_dinv, const int32_t* row_map, float* const* peers, int n_peers,
                 const float* row_scale, int agg_defer_scale, cudaStream_t st, int64_t m_batch_rows, int w_batch_rows,
-                int64_t w_rows_total, int in_f16, int out_f16, int agg_pre) {
+                int64_t w_rows_total, int in_f16, int out_f16, int agg_pre, int a_seg_k0, int a0_cols, const void* A1,
+                int64_t lda1) {
   FG_REQUIRE(!agg_pre || agg_desc, FITGNN_EINVAL, "gemm: agg_pre needs the aggregation descriptors");
+  FG_REQUIRE(!a_seg_k0 || (in_f16 && A1 && a_seg_k0 % tc::BLOCK_K == 0 && a0_cols > 0 && a0_cols <= a_seg_k0 &&
+                           K > a_seg_k0 && !agg_desc && !m_batch_rows),
+             FITGNN_EINVAL, "gemm: a two-segment A needs one fp16 plane per segment and K0 on a k-block boundary");
   FG_REQUIRE(W_lo || in_f16, FITGNN_EINVAL, "gemm: a single-plane W (W_lo = NULL) needs the fp16 operand format");
   FG_REQUIRE(!in_f16 || !A_lo, FITGNN_EINVAL, "gemm: FP16X2 takes ONE fp16 A plane (A_lo must be NULL)");
   FG_REQUIRE(in_f16 || A_lo, FITGNN_EINVAL, "gemm: BF16X3 needs the A_lo plane");
@@ -1311,12 +1322,17 @@ int gemm_bf16x3(const void* A_hi, const void* A_lo, int64_t lda, const void* W_h
   int sms = sm_count() - tuning().sm_reserve;
   if (sms < 2) sms = 2;
   CUtensorMap a_hi, a_lo;
-  FG_TRY(tc::make_map(&a_hi, A_hi, M, K, lda, tc::BLOCK_M));
-  FG_TRY(tc::make_map(&a_lo, A_lo ? A_lo : A_hi, M, K, lda, tc::BLOCK_M));  // unused with a single-plane A
+  if (a_seg_k0) {  // segment 0: A_hi's a0_cols columns, zero-filled to K0; segment 1: A1's K - K0 columns, zero-filled to K
+    FG_TRY(tc::make_map(&a_hi, A_hi, M, a0_cols, lda, tc::BLOCK_M));
+    FG_TRY(tc::make_map(&a_lo, A1, M, K - a_seg_k0, lda1, tc::BLOCK_M));
+  } else {
+    FG_TRY(tc::make_map(&a_hi, A_hi, M, K, lda, tc::BLOCK_M));
+    FG_TRY(tc::make_map(&a_lo, A_lo ? A_lo : A_hi, M, K, lda, tc::BLOCK_M));  // unused with a single-plane A
+  }
   const tc::GatherArgs ga{};
   tc::EpiArgs ea{reinterpret_cast<const unsigned long long*>(agg_desc), agg_dinv, row_map, {}, n_peers, 0, row_scale,
                  agg_defer_scale, m_batch_rows, w_batch_rows, w_rows_total, in_f16 ? 1 : 2, in_f16 ? 1 : 0, out_f16 ? 1 : 0,
-                 W_lo ? 2 : 1, tuning().gemm_prefetch, tuning().gemm_debug};
+                 W_lo ? 2 : 1, tuning().gemm_prefetch, tuning().gemm_debug, a_seg_k0 / tc::BLOCK_K};
   for (int p = 0; p < n_peers; ++p) ea.peers[p] = peers[p];
   if (n_peers > 0) Y = peers[0];  // alignment checks / unused fallbacks refer to a real buffer
   if (row_map && N <= 64 && ldy == (N + 3) / 4 * 4 && tuning().head_bulk) {

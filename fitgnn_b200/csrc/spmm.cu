@@ -1003,18 +1003,39 @@ extern "C" int fitgnn_spmm_symnorm_grouped_f16(const int32_t* rowptr, const int3
 // once and then gathers their rows FG_SPMM_UNROLL at a time.  The sum runs in CSR order as one fmaf chain per element, then
 // ONE correctly rounded division by the count, so results do not depend on out_rows / src_index / the launch shape.
 // Rows of any length are walked in LPR-entry chunks by their own group (no hub split).
+// XH: X is ONE fp16 plane and a lane's unit is a group of 8 halfs (one 16-byte load, two float4 accumulators; nq / nqh count
+// groups), as the fp16 variant of spmm_pipe_kernel.  OUT: fp32, bf16 hi/lo planes or ONE fp16 plane (rounded once,
+// saturating).  concat = 0 (concat form only): the mean half alone, Y[i] = mean, `half` columns.
 // ---------------------------------------------------------------------------------------------------------
 namespace fitgnn {
 
-template <int NV, int LPR, bool ROOT, bool SPLIT>
+template <int OUT, bool XH>
+__device__ __forceinline__ void store_grp(void* Y, void* Ylo, int64_t off, const float4 (&o)[XH ? 2 : 1]) {
+  if constexpr (XH) {
+    static_assert(OUT == IO_F16, "an fp16-plane input is written as an fp16 plane");
+    uint4 pk;
+    pk.x = pack_f16x2_rn(o[0].x, o[0].y);
+    pk.y = pack_f16x2_rn(o[0].z, o[0].w);
+    pk.z = pack_f16x2_rn(o[1].x, o[1].y);
+    pk.w = pack_f16x2_rn(o[1].z, o[1].w);
+    *reinterpret_cast<uint4*>(static_cast<__half*>(Y) + off) = pk;
+  } else {
+    store_row4<OUT>(Y, Ylo, off, o[0]);
+  }
+}
+
+template <int NV, int LPR, bool ROOT, int OUT, bool XH>
 __global__ void __launch_bounds__(SPMM_THREADS, FG_SPMM_MINB)
 spmm_mean_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col, const float* __restrict__ X,
                  int64_t ldx, int nq, int nqh, int64_t root_off, const int32_t* __restrict__ src_index,
                  const float* __restrict__ src_scale, int skip_self, const float* __restrict__ bias, int act,
-                 const int32_t* __restrict__ out_rows, int64_t n_out, void* Y, void* Ylo, int64_t ldy) {
+                 const int32_t* __restrict__ out_rows, int64_t n_out, void* Y, void* Ylo, int64_t ldy, int concat) {
+  static_assert(!(ROOT && XH), "the root form reads the fp32 Z of the first transform");
   constexpr unsigned FULL = 0xffffffffu;
   constexpr int G = 32 / LPR;
   constexpr int U = FG_SPMM_UNROLL;
+  constexpr int EPG = XH ? 8 : 4;  // elements per group
+  constexpr int W4 = XH ? 2 : 1;   // float4 accumulators per group
   constexpr unsigned GMASK = LPR == 32 ? FULL : ((1u << LPR) - 1u);
   const int lane = threadIdx.x & 31;
   const int sub = lane & (LPR - 1);
@@ -1029,9 +1050,9 @@ spmm_mean_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__
   }
   const int64_t root = live ? (src_index ? (int64_t)__ldg(src_index + r) : (int64_t)r) * ldx + root_off : 0;
   for (int q0 = 0; q0 < nqh; q0 += LPR * NV) {
-    float4 acc[NV];
+    Grp<XH> acc[NV];
 #pragma unroll
-    for (int v = 0; v < NV; ++v) acc[v] = make_float4(0.f, 0.f, 0.f, 0.f);
+    for (int v = 0; v < NV; ++v) acc[v] = grp_zero<XH>();
     int cnt = 0;
     for (int e0 = beg; __any_sync(FULL, e0 < end); e0 += LPR) {
       int c = -1;
@@ -1054,19 +1075,21 @@ spmm_mean_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__
           pj[u] = __shfl_sync(FULL, soff, j + u, LPR);
           on[u] = j + u < LPR && ((gm >> (j + u)) & 1u);
         }
-        float4 x[U][NV];
+        Grp<XH> x[U][NV];
 #pragma unroll
         for (int u = 0; u < U; ++u)
 #pragma unroll
           for (int v = 0; v < NV; ++v) {
             const int q = q0 + sub + LPR * v;
-            x[u][v] = (on[u] && q < nq) ? ldg4(X + pj[u] + 4 * q) : make_float4(0.f, 0.f, 0.f, 0.f);
+            x[u][v] = (on[u] && q < nq) ? grp_load<XH>(X, pj[u] + EPG * q) : grp_zero<XH>();
           }
 #pragma unroll
         for (int u = 0; u < U; ++u)
           if (on[u]) {
 #pragma unroll
-            for (int v = 0; v < NV; ++v) fma4(acc[v], wj[u], x[u][v]);
+            for (int v = 0; v < NV; ++v)
+#pragma unroll
+              for (int h = 0; h < W4; ++h) fma4(acc[v].v[h], wj[u], x[u][v].v[h]);
           }
       }
     }
@@ -1076,65 +1099,80 @@ spmm_mean_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__
     for (int v = 0; v < NV; ++v) {
       const int q = q0 + sub + LPR * v;
       if (q >= nqh) continue;
-      float4 o = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (q < nq) {
-        o = acc[v];
-        if (!src_scale && cnt > 0) {
-          o.x = __fdiv_rn(o.x, fc); o.y = __fdiv_rn(o.y, fc); o.z = __fdiv_rn(o.z, fc); o.w = __fdiv_rn(o.w, fc);
+      float4 o[W4];
+#pragma unroll
+      for (int h = 0; h < W4; ++h) {
+        o[h] = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (q < nq) {
+          o[h] = acc[v].v[h];
+          if (!src_scale && cnt > 0) {
+            o[h].x = __fdiv_rn(o[h].x, fc); o[h].y = __fdiv_rn(o[h].y, fc);
+            o[h].z = __fdiv_rn(o[h].z, fc); o[h].w = __fdiv_rn(o[h].w, fc);
+          }
         }
       }
       if (ROOT) {
         const float4 z = ldg4(X + root + 4 * q);
-        o.x += z.x; o.y += z.y; o.z += z.z; o.w += z.w;
+        o[0].x += z.x; o[0].y += z.y; o[0].z += z.z; o[0].w += z.w;
         if (bias) {
           const float4 b = ldg4(bias + 4 * q);
-          o.x += b.x; o.y += b.y; o.z += b.z; o.w += b.w;
+          o[0].x += b.x; o[0].y += b.y; o[0].z += b.z; o[0].w += b.w;
         }
         if (act == FITGNN_ACT_ELU) {
-          o.x = elu1(o.x); o.y = elu1(o.y); o.z = elu1(o.z); o.w = elu1(o.w);
+          o[0].x = elu1(o[0].x); o[0].y = elu1(o[0].y); o[0].z = elu1(o[0].z); o[0].w = elu1(o[0].w);
         }
-        store_row4<SPLIT ? IO_SPLIT : IO_F32>(Y, Ylo, i * ldy + 4 * q, o);
+        store_row4<OUT>(Y, Ylo, i * ldy + 4 * q, o[0]);
       } else {
-        store_row4<SPLIT ? IO_SPLIT : IO_F32>(Y, Ylo, i * ldy + 4 * q, o);
-        const float4 z = q < nq ? ldg4(X + root + 4 * q) : make_float4(0.f, 0.f, 0.f, 0.f);
-        store_row4<SPLIT ? IO_SPLIT : IO_F32>(Y, Ylo, i * ldy + 4 * (int64_t)nqh + 4 * q, z);
+        store_grp<OUT, XH>(Y, Ylo, i * ldy + EPG * q, o);
+        if (concat) {
+          const Grp<XH> z = q < nq ? grp_load<XH>(X, root + EPG * q) : grp_zero<XH>();
+          store_grp<OUT, XH>(Y, Ylo, i * ldy + EPG * (int64_t)nqh + EPG * q, z.v);
+        }
       }
     }
   }
 }
 
-template <int NV, int LPR, bool ROOT>
+template <int NV, int LPR, bool ROOT, int OUT, bool XH>
 static int launch_mean(const int32_t* rowptr, const int32_t* col, const float* X, int64_t ldx, int nq, int nqh,
                        int64_t root_off, const int32_t* src_index, const float* src_scale, int skip_self, const float* bias,
-                       int act, const int32_t* out_rows, int64_t n_out, void* Y, void* Ylo, int64_t ldy, cudaStream_t st) {
+                       int act, const int32_t* out_rows, int64_t n_out, void* Y, void* Ylo, int64_t ldy, int concat,
+                       cudaStream_t st) {
   constexpr int G = 32 / LPR;
   const int64_t blocks = ceil_div(n_out, (int64_t)G * SPMM_WARPS);
   FG_REQUIRE(blocks < (1ll << 31), FITGNN_ERANGE, "spmm_mean: too many rows");
-  if (Ylo)
-    spmm_mean_kernel<NV, LPR, ROOT, true><<<(unsigned)blocks, SPMM_THREADS, 0, st>>>(
-        rowptr, col, X, ldx, nq, nqh, root_off, src_index, src_scale, skip_self, bias, act, out_rows, n_out, Y, Ylo, ldy);
-  else
-    spmm_mean_kernel<NV, LPR, ROOT, false><<<(unsigned)blocks, SPMM_THREADS, 0, st>>>(
-        rowptr, col, X, ldx, nq, nqh, root_off, src_index, src_scale, skip_self, bias, act, out_rows, n_out, Y, Ylo, ldy);
+  spmm_mean_kernel<NV, LPR, ROOT, OUT, XH><<<(unsigned)blocks, SPMM_THREADS, 0, st>>>(
+      rowptr, col, X, ldx, nq, nqh, root_off, src_index, src_scale, skip_self, bias, act, out_rows, n_out, Y, Ylo, ldy, concat);
   FG_LAUNCH_CHECK();
   return FITGNN_OK;
 }
 
-template <bool ROOT>
+// nq / nqh: groups (float4, or 8 halfs with XH) of the input row and of the output half
+template <bool ROOT, int OUT, bool XH>
 static int mean_dispatch(const int32_t* rowptr, const int32_t* col, const float* X, int64_t ldx, int nq, int nqh,
                          int64_t root_off, const int32_t* src_index, const float* src_scale, int skip_self, const float* bias,
-                         int act, const int32_t* out_rows, int64_t n_out, void* Y, void* Ylo, int64_t ldy, void* stream) {
+                         int act, const int32_t* out_rows, int64_t n_out, void* Y, void* Ylo, int64_t ldy, void* stream,
+                         int concat = 1) {
   if (n_out == 0) return FITGNN_OK;
   cudaStream_t st = as_stream(stream);
 #define FG_MEAN(NV, LPR)                                                                                                    \
-  return launch_mean<NV, LPR, ROOT>(rowptr, col, X, ldx, nq, nqh, root_off, src_index, src_scale, skip_self, bias, act,   \
-                                    out_rows, n_out, Y, Ylo, ldy, st)
+  return launch_mean<NV, LPR, ROOT, OUT, XH>(rowptr, col, X, ldx, nq, nqh, root_off, src_index, src_scale, skip_self, bias, \
+                                             act, out_rows, n_out, Y, Ylo, ldy, concat, st)
+  if constexpr (XH) {
+    // (groups of 8 halfs per lane, lanes per row) as the fp16 spmm_dispatch: 64 halfs -> 8 x 1, 128 -> 8 x 2, 256 -> 16 x 2,
+    // 512 per column block beyond
+    if (nqh <= 8) { FG_MEAN(1, 8); }
+    if (nqh <= 16) { FG_MEAN(2, 8); }
+    if (nqh <= 32) { FG_MEAN(2, 16); }
+    FG_MEAN(2, 32);
+  } else {
   // (float4 per lane, lanes per row) from the output half's width, as spmm_dispatch; wider rows loop over 512-column blocks
   if (nqh <= 8) { FG_MEAN(1, 8); }
   if (nqh <= 16) { FG_MEAN(2, 8); }
   if (nqh <= 32) { FG_MEAN(4, 8); }
   if (nqh <= 64) { FG_MEAN(4, 16); }
   FG_MEAN(4, 32);
+  }
 #undef FG_MEAN
 }
 
@@ -1151,8 +1189,11 @@ extern "C" int fitgnn_spmm_mean_concat(const int32_t* rowptr, const int32_t* col
              half, (long long)ldx, (long long)ldy);
   FG_REQUIRE(((uintptr_t)X % 16) == 0 && ((uintptr_t)Y % (Y_lo ? 8 : 16)) == 0 && ((uintptr_t)Y_lo % 8) == 0, FITGNN_EUNSUP,
              "spmm_mean_concat: X must be 16-byte aligned, Y 16-byte (fp32) / 8-byte (planes)");
-  return mean_dispatch<false>(rowptr, col, X, ldx, width / 4, half / 4, 0, src_index, src_scale, skip_self, nullptr,
-                              FITGNN_ACT_NONE, out_rows, n_out, Y, Y_lo, ldy, stream);
+  if (Y_lo)
+    return mean_dispatch<false, IO_SPLIT, false>(rowptr, col, X, ldx, width / 4, half / 4, 0, src_index, src_scale, skip_self,
+                                                 nullptr, FITGNN_ACT_NONE, out_rows, n_out, Y, Y_lo, ldy, stream);
+  return mean_dispatch<false, IO_F32, false>(rowptr, col, X, ldx, width / 4, half / 4, 0, src_index, src_scale, skip_self,
+                                             nullptr, FITGNN_ACT_NONE, out_rows, n_out, Y, Y_lo, ldy, stream);
 }
 
 extern "C" int fitgnn_spmm_mean_root(const int32_t* rowptr, const int32_t* col, const float* Z, int64_t ldz, int width,
@@ -1170,6 +1211,42 @@ extern "C" int fitgnn_spmm_mean_root(const int32_t* rowptr, const int32_t* col, 
                  (!bias || ((uintptr_t)bias % 16) == 0),
              FITGNN_EUNSUP, "spmm_mean_root: Z / bias must be 16-byte aligned, Y 16-byte (fp32) / 8-byte (planes)");
   FG_REQUIRE(act == FITGNN_ACT_NONE || act == FITGNN_ACT_ELU, FITGNN_EINVAL, "spmm_mean_root: unknown act %d", act);
-  return mean_dispatch<true>(rowptr, col, Z, ldz, width / 4, width / 4, root_off, src_index, src_scale, skip_self, bias, act,
-                             out_rows, n_out, Y, Y_lo, ldy, stream);
+  if (Y_lo)
+    return mean_dispatch<true, IO_SPLIT, false>(rowptr, col, Z, ldz, width / 4, width / 4, root_off, src_index, src_scale,
+                                                skip_self, bias, act, out_rows, n_out, Y, Y_lo, ldy, stream);
+  return mean_dispatch<true, IO_F32, false>(rowptr, col, Z, ldz, width / 4, width / 4, root_off, src_index, src_scale, skip_self,
+                                            bias, act, out_rows, n_out, Y, Y_lo, ldy, stream);
+}
+
+// ---- the mean aggregation on fp16 planes (PackedForward(precision="fp16x2" / "fp16") for SAGE; include/fitgnn.h) --------
+extern "C" int fitgnn_spmm_mean_f16(const int32_t* rowptr, const int32_t* col, const void* X, int64_t ldx, int width, int half,
+                                    const int32_t* src_index, int skip_self, int concat, const int32_t* out_rows, int64_t n_out,
+                                    void* Y, int64_t ldy, void* stream) {
+  FG_REQUIRE(rowptr && col && X && Y, FITGNN_EINVAL, "spmm_mean_f16: null pointer");
+  FG_REQUIRE(n_out >= 0 && width > 0 && half >= width, FITGNN_EINVAL, "spmm_mean_f16: n_out=%lld width=%d half=%d",
+             (long long)n_out, width, half);
+  FG_REQUIRE(width % 8 == 0 && half % 8 == 0 && ldx % 8 == 0 && ldy % 8 == 0 && ldx >= width &&
+                 ldy >= (concat ? 2 : 1) * (int64_t)half,
+             FITGNN_EUNSUP, "spmm_mean_f16: width (%d), half (%d), ldx (%lld), ldy (%lld) must be multiples of 8, ldx >= width, "
+             "ldy >= %s", width, half, (long long)ldx, (long long)ldy, concat ? "2 * half" : "half");
+  FG_REQUIRE(((uintptr_t)X % 16) == 0 && ((uintptr_t)Y % 16) == 0, FITGNN_EUNSUP, "spmm_mean_f16: planes must be 16-byte aligned");
+  return mean_dispatch<false, IO_F16, true>(rowptr, col, static_cast<const float*>(X), ldx, width / 8, half / 8, 0, src_index,
+                                            nullptr, skip_self, nullptr, FITGNN_ACT_NONE, out_rows, n_out, Y, nullptr, ldy,
+                                            stream, concat ? 1 : 0);
+}
+
+extern "C" int fitgnn_spmm_mean_root_f16(const int32_t* rowptr, const int32_t* col, const float* Z, int64_t ldz, int width,
+                                         int64_t root_off, const int32_t* src_index, int skip_self, const float* bias, int act,
+                                         const int32_t* out_rows, int64_t n_out, void* Y, int64_t ldy, void* stream) {
+  FG_REQUIRE(rowptr && col && Z && Y, FITGNN_EINVAL, "spmm_mean_root_f16: null pointer");
+  FG_REQUIRE(n_out >= 0 && width > 0 && root_off >= 0, FITGNN_EINVAL, "spmm_mean_root_f16: n_out=%lld width=%d root_off=%lld",
+             (long long)n_out, width, (long long)root_off);
+  FG_REQUIRE(width % 4 == 0 && root_off % 4 == 0 && ldz % 4 == 0 && ldy % 4 == 0 && ldy >= width && root_off + width <= ldz,
+             FITGNN_EUNSUP, "spmm_mean_root_f16: width (%d), root_off (%lld), ldz (%lld), ldy (%lld): multiples of 4, "
+             "root_off + width <= ldz", width, (long long)root_off, (long long)ldz, (long long)ldy);
+  FG_REQUIRE(((uintptr_t)Z % 16) == 0 && ((uintptr_t)Y % 8) == 0 && (!bias || ((uintptr_t)bias % 16) == 0), FITGNN_EUNSUP,
+             "spmm_mean_root_f16: Z / bias must be 16-byte aligned, Y 8-byte");
+  FG_REQUIRE(act == FITGNN_ACT_NONE || act == FITGNN_ACT_ELU, FITGNN_EINVAL, "spmm_mean_root_f16: unknown act %d", act);
+  return mean_dispatch<true, IO_F16, false>(rowptr, col, Z, ldz, width / 4, width / 4, root_off, src_index, nullptr, skip_self,
+                                            bias, act, out_rows, n_out, Y, nullptr, ldy, stream);
 }

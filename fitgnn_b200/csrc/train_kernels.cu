@@ -18,7 +18,8 @@ int gemm_bf16x3(const void* A_hi, const void* A_lo, int64_t lda, const void* W_h
                 const float* bias, int64_t M, int K, int N, int act, int head, float* Y, void* Y_lo, int64_t ldy,
                 const uint64_t* agg_desc, const float* agg_dinv, const int32_t* row_map, float* const* peers, int n_peers,
                 const float* row_scale, int agg_defer_scale, cudaStream_t st, int64_t m_batch_rows, int w_batch_rows,
-                int64_t w_rows_total, int in_f16 = 0, int out_f16 = 0, int agg_pre = 0);
+                int64_t w_rows_total, int in_f16 = 0, int out_f16 = 0, int agg_pre = 0, int a_seg_k0 = 0,
+                int a0_cols = 0, const void* A1 = nullptr, int64_t lda1 = 0);
 
 namespace {
 

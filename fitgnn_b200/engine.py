@@ -20,8 +20,14 @@ transform-first Z = X·[W_l ; W_r]^T on the de-duplicated rows followed by mean 
 aggregate-first; the last one on the output rows only; then the head.  The pack's CSR is used as is and its one self entry
 per row is the root, not a neighbour (skip_self).  A pack collapses the self-loop edges of its input into that single entry,
 so on a graph with self-loop edges the pack result differs from PyG's SAGEConv, which counts such an edge as a neighbour;
-the subgraphs the reference builds have none.  bf16x3 or fp32 only (the fp16 precisions run bf16x3, as for packs that are
-not eligible for the fused schedule); the fused aggregation is not built for SAGE.
+the subgraphs the reference builds have none.  The fused aggregation is not built for SAGE.
+SAGE under precision 'fp16x2' / 'fp16' (L >= 2, with the head, hidden % 8 == 0 and >= 32, as GCN's classic fp16 schedule;
+other SAGE models run bf16x3): the hidden state is ONE fp16 plane.  Layer 0 as above on bf16 planes, but its transform
+(aggregate-first) or the root form (transform-first) writes the fp16 plane; layers >= 1 aggregate fp16 -> fp16 (the mean alone)
+and ONE transform reads k-blocks [0, K0) from the mean plane and the rest from h itself (ops.gemm_f16_2seg: no concatenated
+operand, no copy of the root rows), against [W_l | 0 | W_r] with K0 = hidden rounded up to 64, as fp16 hi/lo weights ('fp16x2')
+or one fp16 plane ('fp16'); a last layer on a row subset writes [mean | root] of those rows instead and runs ops.gemm_f16; the
+head reads the fp16 plane with fp16 hi/lo weights.
 """
 from __future__ import annotations
 
@@ -210,27 +216,40 @@ class PackedForward:
         from .autograd import sage_weight_cat
         if fuse_aggregate is True:
             raise ValueError("fuse_aggregate=True: the fused aggregation is not built for SAGEConv models")
+        w_single = self.w_single
+        w0 = sd["conv.0.lin_l.weight"]
+        # the fp16 schedule (module docstring) under GCN's classic-fp16 eligibility; any other model runs bf16x3
+        self.sage_f16 = bool(self.f16_hidden and self.L >= 2 and self.with_head and w0.shape[0] % 8 == 0 and w0.shape[0] >= 32)
         self.f16_hidden = self.w_single = self.f16_classic = self.f16_layer0 = self.conv_fused = False
         self.apack, self._blk, self._head_map = None, None, None
         self.fused_layer0 = False
         self.prof, self.launches, self._nnz_cache = None, 0, {}
-        w0 = sd["conv.0.lin_l.weight"]
         self.F, self.H = w0.shape[1], w0.shape[0]
         assert self.H % 4 == 0, "hidden width must be a multiple of 4"
         self.Fp, self.Hp = self._kpad(self.F), self._kpad(self.H)
         self.transform_first = self.F > self.H
+        # fp16 layers >= 1: each weight half starts on a k-block (64) boundary, so the mean plane and h are the two segments of
+        # the transform's A operand (ops.gemm_f16_2seg) and the concat form of the last layer uses the same weights
+        self.K0 = (self.H + 63) // 64 * 64
         self.W, self.b = [], []
         for i in range(self.L):
             wl = sd[f"conv.{i}.lin_l.weight"].detach().to(**f32)
             wr = sd[f"conv.{i}.lin_r.weight"].detach().to(**f32)
             if i == 0 and self.transform_first:
                 w = torch.cat([wl, wr], 0)  # [2H, F]: Z = X·[W_l ; W_r]^T
+            elif i > 0 and self.sage_f16:
+                w = sage_weight_cat(wl, wr, self.K0)  # fp16 planes [H, 2 K0]: one plane under 'fp16', hi/lo under 'fp16x2'
+                self.W.append(ops.split_f16(w, lo=not w_single))
+                self.b.append(sd[f"conv.{i}.lin_l.bias"].detach().to(**f32).contiguous())
+                continue
             else:
                 w = sage_weight_cat(wl, wr, self.Fp if i == 0 else self.Hp)  # [H, 2 half]: [mean x | x]·[W_l | W_r]^T
             self.W.append(self._prep_weight(w))
             self.b.append(sd[f"conv.{i}.lin_l.bias"].detach().to(**f32).contiguous())
         if self.with_head:
-            self.Wl = self._prep_weight(sd["lt1.weight"].detach().to(**f32))
+            wl = sd["lt1.weight"].detach().to(**f32)
+            # the fp16 schedule's head keeps fp16 hi/lo weights
+            self.Wl = ops.split_f16(wl.contiguous(), ldo=self._kpad(self.H)) if self.sage_f16 else self._prep_weight(wl)
             self.bl = sd["lt1.bias"].detach().to(**f32).contiguous()
             self.C = sd["lt1.weight"].shape[0]
         self._select_rows(rows)
@@ -240,7 +259,7 @@ class PackedForward:
             self.out_map = out_map.to(device=self.pack.device, dtype=torch.int32).contiguous()
             assert self.out_map.numel() == self.n_out
 
-    def _mean(self, name, fn, width, in_cols, out_cols, src_index, last, n_src_rows, out_elem):
+    def _mean(self, name, fn, width, in_cols, out_cols, src_index, last, n_src_rows, out_elem, in_elem=4):
         """One mean-aggregation launch; bytes: rowptr + col, every distinct source row once (in_cols wide: the root form
         reads both halves of Z), the output rows, gid and the row selection."""
         p = self.pack
@@ -249,7 +268,7 @@ class PackedForward:
             r = self.out_rows.long() if (last and self.out_rows is not None) else None
             self._nnz_cache[key] = p.nnz if r is None else int((p.rowptr.long()[r + 1] - p.rowptr.long()[r]).sum())
         r_out = self.n_out if last else p.n_rows
-        nb = 4 * (r_out + 1) + 4 * self._nnz_cache[key] + 4 * n_src_rows * in_cols + out_elem * r_out * out_cols
+        nb = 4 * (r_out + 1) + 4 * self._nnz_cache[key] + in_elem * n_src_rows * in_cols + out_elem * r_out * out_cols
         nb += 4 * p.n_rows if src_index is not None else 0
         nb += 4 * r_out if (last and self.out_rows is not None) else 0
         self.launches += 1
@@ -260,6 +279,8 @@ class PackedForward:
         bf = self.precision == ops.GEMM_BF16X3
         X = self.pad_features(X)
         gid0 = None if packed else p.gid
+        if self.sage_f16:
+            return self._forward_sage_f16(X, gid0, out)
         H, Fp, Hp = self.H, self.Fp, self.Hp
         h = None
         for i in range(self.L):
@@ -282,6 +303,43 @@ class PackedForward:
             to_head = bf and last and self.with_head and H % 8 == 0
             h = self._gemm(A, self.W[i], self.b[i], ops.ACT_ELU, N=H, K=2 * half, name=f"gemm{i}", split_out=to_head)
         return self._finish(h, out, X.device)
+
+    def _forward_sage_f16(self, X, gid0, out):
+        """The SAGE classic schedule with the hidden state as ONE fp16 plane (precision 'fp16x2' / 'fp16'; module docstring)."""
+        p = self.pack
+        H, Fp, K0, M = self.H, self.Fp, self.K0, p.n_rows
+        if self.transform_first:  # bf16x3 Z on the de-duplicated rows, then mean + root + bias + ELU into the fp16 plane
+            A = ops.split_bf16(X)
+            self.launches += 1
+            Z = self._gemm(A, self.W[0], None, ops.ACT_NONE, N=2 * H, K=Fp, name="gemm0_unique_rows")
+            h = self._mean("mean0", lambda: ops.spmm_mean_root_f16(p.rowptr, p.col, Z, H, H, gid0, True, self.b[0], ops.ACT_ELU),
+                           H, 2 * H, H, gid0, False, Z.shape[0], 2)
+        else:  # bf16 hi/lo [mean x | x], then the transform writes the fp16 plane
+            A = self._mean("mean0", lambda: ops.spmm_mean_concat(p.rowptr, p.col, X, Fp, Fp, gid0, None, True, split=True),
+                           Fp, Fp, 2 * Fp, gid0, False, X.shape[0] if gid0 is not None else M, 4)
+            self.launches += 1
+            h = self._timed("gemm0", lambda: ops.gcn_transform_aggregate_f16(A, self.W[0], self.b[0], ops.ACT_ELU, None, None,
+                                                                             K=2 * Fp, N=H),
+                            nbytes=4 * M * 2 * Fp + 4 * 2 * Fp * H + 2 * M * H, flops=2 * M * 2 * Fp * H)
+        for i in range(1, self.L):
+            last = i == self.L - 1
+            src = h
+            if last and self.out_rows is not None:  # [mean | root] of the output rows only, then one transform
+                n = self.n_out
+                A = self._mean(f"mean{i}", lambda: ops.spmm_mean_f16(p.rowptr, p.col, src, H, K0, None, True, self.out_rows,
+                                                                     concat=True),
+                               H, H, 2 * K0, None, True, M, 2, in_elem=2)
+                self.launches += 1
+                h = self._timed(f"gemm{i}", lambda: ops.gemm_f16(A, self.W[i], self.b[i], ops.ACT_ELU, out_f16=True, K=2 * K0, N=H),
+                                nbytes=2 * n * 2 * K0 + 4 * 2 * K0 * H + 2 * n * H, flops=2 * n * 2 * K0 * H)
+            else:  # every pack row is an output row: the transform reads the mean plane and h itself (no root copy)
+                Mn = self._mean(f"mean{i}", lambda: ops.spmm_mean_f16(p.rowptr, p.col, src, H, H, None, True),
+                                H, H, H, None, last, M, 2, in_elem=2)
+                self.launches += 1
+                h = self._timed(f"gemm{i}", lambda: ops.gemm_f16_2seg(Mn, src, self.W[i], K0, self.b[i], ops.ACT_ELU, out_f16=True,
+                                                                      N=H),
+                                nbytes=2 * M * 2 * H + 4 * (K0 + H) * H + 2 * M * H, flops=2 * M * (K0 + H) * H)
+        return self._head_f16(h, out, X.device)
 
     # -- per-kernel timing for the roofline report (CUDA events on the launching stream) ---------
     def enable_profile(self, on=True):
@@ -657,6 +715,11 @@ class PackedForward:
             self.launches += 1
             h = self._timed(f"gemm{i}", lambda: ops.gemm_f16(A, self.W[i], self.b[i], ops.ACT_ELU, out_f16=True, K=H, N=H),
                             nbytes=2 * n_rows * H + 4 * H * H + 2 * n_rows * H, flops=2 * n_rows * H * H)
+        return self._head_f16(h, out, X.device)
+
+    def _head_f16(self, h, out, device):
+        """Head of the classic fp16 schedules on the last hidden state h (ONE fp16 plane, the output rows)."""
+        H = self.H
         n = self.n_out
         self.launches += 1
         nb = 2 * n * H + 4 * H * self.C + 4 * n * self.C
@@ -667,7 +730,7 @@ class PackedForward:
             return out
         view = None
         if out is None:
-            out = torch.empty(n, ops.pad4(self.C), dtype=torch.float32, device=X.device)
+            out = torch.empty(n, ops.pad4(self.C), dtype=torch.float32, device=device)
         if out.shape[1] != self.C:
             view = out[:, : self.C]
         self._timed("head", lambda: ops.gemm_f16(h, self.Wl, self.bl, ops.ACT_NONE, self.head, out=out, K=H, N=self.C),

@@ -114,6 +114,36 @@ def spmm_mean_root(rowptr, col, Z, width, root_off=None, src_index=None, src_sca
     return out
 
 
+def spmm_mean_f16(rowptr, col, X, width=None, half=None, src_index=None, skip_self=False, out_rows=None, concat=False,
+                  out=None):
+    """spmm_mean_concat on fp16 planes (fitgnn_spmm_mean_f16): X one fp16 plane, the result one fp16 plane [n_out, half]
+    (the mean alone) or, concat=True, [n_out, 2*half] = [mean | root]; fp32 sums, one saturating rounding."""
+    assert X.dtype == torch.float16 and X.dim() == 2
+    width = X.shape[1] if width is None else width
+    half = width if half is None else half
+    n_out = out_rows.numel() if out_rows is not None else rowptr.numel() - 1
+    if out is None:
+        out = torch.empty(n_out, 2 * half if concat else half, dtype=torch.float16, device=X.device)
+    check(lib().fitgnn_spmm_mean_f16(ptr(rowptr), ptr(col), ptr(X), X.stride(0), width, half, ptr(src_index),
+                                     int(bool(skip_self)), int(bool(concat)), ptr(out_rows), n_out, ptr(out), out.stride(0),
+                                     stream_ptr()))
+    return out
+
+
+def spmm_mean_root_f16(rowptr, col, Z, width, root_off=None, src_index=None, skip_self=False, bias=None, act=ACT_NONE,
+                       out_rows=None, out=None):
+    """spmm_mean_root whose result is ONE fp16 plane [n_out, width] (fitgnn_spmm_mean_root_f16); Z stays fp32."""
+    assert Z.dtype == torch.float32 and Z.dim() == 2
+    root_off = width if root_off is None else root_off
+    n_out = out_rows.numel() if out_rows is not None else rowptr.numel() - 1
+    if out is None:
+        out = torch.empty(n_out, width, dtype=torch.float16, device=Z.device)
+    check(lib().fitgnn_spmm_mean_root_f16(ptr(rowptr), ptr(col), ptr(Z), Z.stride(0), width, root_off, ptr(src_index),
+                                          int(bool(skip_self)), ptr(bias), act, ptr(out_rows), n_out, ptr(out), out.stride(0),
+                                          stream_ptr()))
+    return out
+
+
 def spmm_symnorm(rowptr, col, dinv, X, width=None, src_index=None, bias=None, act=ACT_NONE, out_rows=None,
                  out=None, split=False, hubs=None):
     """Y = act(Â·X[src_index] + bias) on the rows `out_rows` (all rows when None).
@@ -608,6 +638,24 @@ def gemm_f16(A, W, bias=None, act=ACT_NONE, head=HEAD_IDENTITY, row_scale=None, 
                           device=A.device)
     check(lib().fitgnn_gemm_f16(ptr(A), A.stride(0), ptr(w_hi), ptr(w_lo), w_hi.stride(0), ptr(row_scale), ptr(bias), M, K, N,
                                 act, head, ptr(out), out.stride(0), int(out_f16), ptr(row_map), stream_ptr()))
+    return out
+
+
+def gemm_f16_2seg(A0, A1, W, K0, bias=None, act=ACT_NONE, out_f16=False, a0_cols=None, K=None, N=None):
+    """act(A·W^T + bias) with A = [A0 | 0 | A1]: k-blocks [0, K0) read the fp16 plane A0 (a0_cols columns, zero beyond), the
+    rest the fp16 plane A1 (K - K0 columns; K defaults to K0 + A1's width) (fitgnn_gemm_f16_2seg).  W = fp16 (hi, lo) planes or
+    (hi, None).  out_f16: the result as one fp16 plane."""
+    w_hi, w_lo = W
+    assert A0.dtype == torch.float16 and A1.dtype == torch.float16 and w_hi.dtype == torch.float16
+    M = A0.shape[0]
+    assert A1.shape[0] == M
+    a0_cols = A0.shape[1] if a0_cols is None else a0_cols
+    K = K0 + A1.shape[1] if K is None else K
+    N = w_hi.shape[0] if N is None else N
+    out = torch.empty(M, N if (out_f16 or N % 4 == 0) else pad4(N), dtype=torch.float16 if out_f16 else torch.float32,
+                      device=A0.device)
+    check(lib().fitgnn_gemm_f16_2seg(ptr(A0), A0.stride(0), a0_cols, K0, ptr(A1), A1.stride(0), ptr(w_hi), ptr(w_lo),
+                                     w_hi.stride(0), ptr(bias), M, K, N, act, ptr(out), out.stride(0), int(out_f16), stream_ptr()))
     return out
 
 

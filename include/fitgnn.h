@@ -360,6 +360,28 @@ int fitgnn_gemm_f16_head_rows_peers(const void* A, int64_t lda, const void* W_hi
                                     const float* bias, int64_t M, int K, int N, int act, int head,
                                     const int32_t* row_map, float* const* host_peer_bases, int n_peers,
                                     int64_t ldy, void* stream);
+/* SAGEConv on the fp16 hidden state (PackedForward(precision="fp16x2" / "fp16") for a SAGE state_dict):
+ *   fitgnn_spmm_mean_f16: the mean aggregation of fitgnn_spmm_mean_concat with X and Y ONE fp16 plane each (ldx / ldy in
+ *     elements; width, half, ldx, ldy multiples of 8, 16-byte aligned planes).  One 16-byte load of 8 halfs per lane and source
+ *     row, fp32 sums in CSR order, one division, one saturating rounding.  concat != 0: Y[i] = [mean | root] as the concat form
+ *     (ldy >= 2*half); concat = 0: the mean alone, Y[i] = mean, columns [width, half) zero (ldy >= half).  skip_self, src_index
+ *     and out_rows as fitgnn_spmm_mean_concat (no src_scale); results are bit-identical across out_rows / src_index.
+ *   fitgnn_spmm_mean_root_f16: fitgnn_spmm_mean_root (fp32 Z, no src_scale) whose output is ONE fp16 plane [n_out, ldy].
+ *   fitgnn_gemm_f16_2seg: fitgnn_gemm_f16 (no row scale, head or row map) whose A operand is two fp16 planes side by side in K:
+ *     columns [0, K0) are A0 (a0_cols <= K0 columns of pitch lda0, zero beyond), columns [K0, K) are A1 (K - K0 columns of
+ *     pitch lda1).  K0 is a multiple of 64 (the k-block).  Neither plane is read beyond its width.  Both planes have M rows.
+ *     With A0 = the mean plane and A1 = the hidden state itself this is lin_l(mean h) + lin_r(h) against
+ *     W = [W_l | 0 | W_r] (K0 = hidden rounded up to 64) without a concatenated operand.  Bit-identical to fitgnn_gemm_f16 on
+ *     the materialised [A0 | 0 | A1]: same plans, same MMAs in the same order. */
+int fitgnn_spmm_mean_f16(const int32_t* rowptr, const int32_t* col, const void* X, int64_t ldx, int width, int half,
+                         const int32_t* src_index, int skip_self, int concat, const int32_t* out_rows, int64_t n_out, void* Y,
+                         int64_t ldy, void* stream);
+int fitgnn_spmm_mean_root_f16(const int32_t* rowptr, const int32_t* col, const float* Z, int64_t ldz, int width,
+                              int64_t root_off, const int32_t* src_index, int skip_self, const float* bias, int act,
+                              const int32_t* out_rows, int64_t n_out, void* Y, int64_t ldy, void* stream);
+int fitgnn_gemm_f16_2seg(const void* A0, int64_t lda0, int a0_cols, int K0, const void* A1, int64_t lda1, const void* W_hi,
+                         const void* W_lo, int64_t ldw, const float* bias, int64_t M, int K, int N, int act, void* Y,
+                         int64_t ldy, int out_f16, void* stream);
 int fitgnn_gcn_transform_aggregate_f16(int in_f16, const void* A_hi, const void* A_lo, int64_t lda, const void* W_hi,
                                        const void* W_lo, int64_t ldw, const float* bias, int64_t M, int K, int N,
                                        int act, const uint64_t* agg_desc, const float* dinv, int defer_row_scale,

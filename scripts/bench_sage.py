@@ -1,16 +1,21 @@
 """SAGEConv on the products-shaped workload of bench.py: ogbn-products-shaped synthetic graph (planted partition, ratio 0.5,
 mode 'none'), F = 100, hidden 512, C = 47, a 2-layer SAGE model (seeded weights with PyG's keys) + lt1 + log_softmax,
-run over the whole pack by PackedForward.  Prints one JSON line:
+run over the whole pack by PackedForward, in every precision given with --precision (bf16x3, fp16x2, fp16; repeatable,
+default bf16x3).  Prints one JSON line with, per precision:
 
-  * step_ms: forward time per step (CUDA events around `--steps` forwards after `--warmup` untimed ones);
+  * step_ms: forward time per step — the median of `--rounds` blocks of `--steps` forwards (CUDA events), after `--warmup`
+    untimed ones; the blocks of the precisions alternate, so all of them see the same state of a shared host;
   * kernels: per launch CUDA-event time, algorithmic bytes / FLOPs, and the share of the least time the hardware could
     take — max(bytes / 7.7 TB/s, tensor work / 2,250 TFLOP/s), the HGX B200 data-sheet figures per GPU — naming which of
-    the two bounds it.  bf16x3 issues three bf16 MMAs per product, so its tensor work is 3x the algorithmic FLOPs;
+    the two bounds it.  Tensor work = MMAs per product x algorithmic FLOPs: 3 for bf16x3 operands (the first layer of every
+    precision), 2 for an fp16 plane against fp16 hi/lo weights (fp16x2, and the head of both fp16 precisions), 1 for one
+    fp16 weight plane (fp16, layers >= 1);
   * parity: logits of a seeded sample of subgraphs against the torch-CPU SAGE restatement (tests/sage_oracle.py) on those
     subgraphs alone; the run aborts above 1e-3 relative;
   * gpu: card name, power limit and max SM clock, read in the same run.
 
-Usage: python scripts/bench_sage.py [--steps 10] [--warmup 3] [--workload products|products-small] [--json-out PATH]
+Usage: python scripts/bench_sage.py [--precision bf16x3 --precision fp16 ...] [--steps 10] [--rounds 3] [--warmup 3]
+       [--workload products|products-small] [--json-out PATH]
 """
 from __future__ import annotations
 
@@ -43,15 +48,24 @@ def gpu_info():
         return {"name": torch.cuda.get_device_name(0), "power_limit": None, "error": repr(e)}
 
 
-def kernel_table(prof):
+def mmas_per_product(name, precision):
+    """MMAs the launch issues per product (0: not a tensor-core launch)."""
+    if not (name.startswith("gemm") or name == "head"):
+        return 0
+    if precision == "bf16x3" or name.startswith("gemm0"):
+        return 3
+    return 1 if (precision == "fp16" and name != "head") else 2
+
+
+def kernel_table(prof, precision):
     out = {}
     for name, r in prof.items():
         s = r["ms"] * 1e-3
-        tensor = 3 * r["flops"] if name.startswith("gemm") or name == "head" else 0
-        t_mem, t_tc = r["bytes"] / (HBM_TBS * 1e12), tensor / (BF16_TFLOPS * 1e12)
+        mma = mmas_per_product(name, precision)
+        t_mem, t_tc = r["bytes"] / (HBM_TBS * 1e12), mma * r["flops"] / (BF16_TFLOPS * 1e12)
         out[name] = {"ms": r["ms"], "launches": r["launches"], "algo_GB": r["bytes"] / 1e9,
                      "algo_TFLOP": r["flops"] / 1e12, "GBps": r["bytes"] / s / 1e9, "TFLOPs": r["flops"] / s / 1e12,
-                     "bound": "hbm" if t_mem >= t_tc else "tensor (bf16x3: 3 MMAs per product)",
+                     "mmas_per_product": mma, "bound": "hbm" if t_mem >= t_tc else f"tensor ({mma} MMAs per product)",
                      "share_of_peak": max(t_mem, t_tc) / s}
     return out
 
@@ -83,11 +97,14 @@ def parity(fg, so, fo, ei, part, X, sd, logits, core_gid, n_sub, k):
 def main():
     p = argparse.ArgumentParser()
     p.add_argument("--steps", type=int, default=10)
+    p.add_argument("--rounds", type=int, default=3)
     p.add_argument("--warmup", type=int, default=3)
+    p.add_argument("--precision", action="append", choices=["bf16x3", "fp16x2", "fp16"])
     p.add_argument("--workload", default="products", choices=sorted(SHAPES))
     p.add_argument("--parity-subgraphs", type=int, default=512)
     p.add_argument("--json-out", default=None)
     a = p.parse_args()
+    precisions = list(dict.fromkeys(a.precision or ["bf16x3"]))
     if not torch.cuda.is_available():
         raise SystemExit("bench_sage: needs a CUDA device (there is no CPU measurement)")
     import fitgnn_b200 as fg
@@ -102,29 +119,40 @@ def main():
     X = fg.synth.features(n, F, seed=0, device=dev)
     sd = {k_: v.to(dev) for k_, v in so.init_state_dict(F, H, C, seed=0).items()}
     pack = fg.build_pack(ei, part, k, "none")
-    fwd = fg.PackedForward(pack, sd, head="log_softmax", rows="core", precision="bf16x3")
-    for _ in range(max(1, a.warmup)):
-        out = fwd(X)
+    fwds = {pr: fg.PackedForward(pack, sd, head="log_softmax", rows="core", precision=pr) for pr in precisions}
+    outs = {}
+    for pr, fwd in fwds.items():
+        for _ in range(max(1, a.warmup)):
+            outs[pr] = fwd(X)
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
-    for _ in range(a.steps):
-        out = fwd(X)
-    e1.record()
-    torch.cuda.synchronize()
-    step_ms = e0.elapsed_time(e1) / a.steps
-    fwd.enable_profile(True)  # per-kernel events in separate passes: the event records stay out of the step time
-    for _ in range(a.steps):
-        fwd(X)
-    torch.cuda.synchronize()
-    kernels = kernel_table(fwd.profile_summary())
-    fwd.enable_profile(False)
+    blocks = {pr: [] for pr in precisions}
+    for _ in range(max(1, a.rounds)):
+        for pr, fwd in fwds.items():
+            e0.record()
+            for _ in range(a.steps):
+                outs[pr] = fwd(X)
+            e1.record()
+            torch.cuda.synchronize()
+            blocks[pr].append(e0.elapsed_time(e1) / a.steps)
+    results = {}
+    for pr, fwd in fwds.items():
+        fwd.enable_profile(True)  # per-kernel events in separate passes: the event records stay out of the step time
+        for _ in range(a.steps):
+            fwd(X)
+        torch.cuda.synchronize()
+        kernels = kernel_table(fwd.profile_summary(), pr)
+        fwd.enable_profile(False)
+        step_ms = float(np.median(blocks[pr]))
+        results[pr] = {"step_ms": step_ms, "step_ms_blocks": blocks[pr], "nodes_per_s": n / (step_ms * 1e-3),
+                       "fp16_schedule": bool(getattr(fwd, "sage_f16", False)), "kernels": kernels,
+                       "sum_kernel_ms": sum(r["ms"] for r in kernels.values()),
+                       "sum_algo_GB": sum(r["algo_GB"] for r in kernels.values()),
+                       "parity": parity(fg, so, fo, ei, part, X, sd, outs[pr], pack.core_gid, a.parity_subgraphs, k)}
     line = {"bench": "sage_products", "workload": f"{a.workload}: {n} nodes, {e_und} undirected edges, planted partition "
                                                   f"ratio 0.5 (k={k}), mode none, F={F}, 2-layer SAGEConv hidden={H}, C={C}",
-            "precision": "bf16x3", "steps": a.steps, "warmup": a.warmup, "step_ms": step_ms,
-            "nodes_per_s": n / (step_ms * 1e-3), "kernels": kernels, "sum_kernel_ms": sum(r["ms"] for r in kernels.values()),
+            "precisions": precisions, "steps": a.steps, "rounds": a.rounds, "warmup": a.warmup, "results": results,
             "pack": {"rows": pack.n_rows, "nnz": pack.nnz, "subgraphs": pack.n_sub},
-            "parity": parity(fg, so, fo, ei, part, X, sd, out, pack.core_gid, a.parity_subgraphs, k),
             "gpu": gpu_info(), "peaks": {"hbm_TBps": HBM_TBS, "bf16_dense_TFLOPs": BF16_TFLOPS, "source": "data sheet"}}
     s = json.dumps(line)
     print(s)
